@@ -3,9 +3,15 @@
 bench.py - throughput of the shift-invariant NMF multiplicative-update (MU) iteration.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload cfg2|cfg3|...]
+                    [--dump-outputs DIR]
 
 A "step" is one batch MU iteration (H update, W update; tnmf/TransformInvariantNMF.py:334-346 of the
 reference) over a synthetic batch.  The metric is BASELINE.json's: sample-iterations per second.
+
+`--dump-outputs DIR` (own arm) writes W and H as they stand after the last timed step to DIR/W.npy and DIR/H.npy
+(rank 0's samples), H as a fixed sample DIR/H_sample.npy where all of it would exceed 64 MB (see `dump_outputs`).  The
+batch and the start values of W and H come from seeded generators of this script, so with the same arguments two
+builds of the library start from the same numbers and can be compared output for output.
 
   * own arm (`--impl b200`): the hand-written sm_100a kernels of libtnmf_b200.so driven through
     `tnmf_b200.TransformInvariantNMF`.  `value` is measured with the batch resident in HBM (CUDA events, max over
@@ -311,6 +317,42 @@ def measure_cfg3(nmf_cls, device, args, world, rank, dist):
     return out
 
 
+DUMP_BYTES = 64 << 20           # most that --dump-outputs writes
+H_SAMPLE = 1 << 22              # elements of H kept when all of it would not fit
+
+
+def seed_start_values(nmf, device, rank):
+    """Overwrite the library's random start values with ones drawn here (1 - U[0, 1), W normalised over its shift axes
+    like the facade does): they then depend neither on how a build lays out H nor on the order it draws in.  W is the
+    same on every rank, H differs per rank like the samples do."""
+    import torch
+    W, H = nmf.W_device, nmf.H_device
+    gen = torch.Generator(device=device)
+    gen.manual_seed(99)
+    W0 = 1 - torch.rand(W.shape, dtype=W.dtype, device=device, generator=gen)
+    W.copy_(W0 / W0.sum(dim=nmf._axes_W_normalization, keepdim=True))  # pylint: disable=protected-access
+    gen.manual_seed(5678 + rank)
+    H.copy_(1 - torch.rand(H.shape, dtype=H.dtype, device=device, generator=gen))
+    torch.cuda.empty_cache()        # the buffers the steps allocate are then placed as if the temporaries never existed
+
+
+def dump_outputs(out_dir, be, W, H):
+    """W and H as .npy files in their own dtype.  An H whose bytes together with W's exceed DUMP_BYTES is written as
+    H_sample.npy: its elements at the flat C-order indices sorted(numpy.random.default_rng(0).choice(H.numel(),
+    H_SAMPLE, replace=False)), the same indices on every run with the same arguments."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for stale in ('H.npy', 'H_sample.npy'):           # a run with other arguments may have left the other form
+        if os.path.exists(os.path.join(out_dir, stale)):
+            os.remove(os.path.join(out_dir, stale))
+    np.save(os.path.join(out_dir, 'W.npy'), be.to_ndarray(W))
+    if (W.numel() + H.numel()) * H.element_size() <= DUMP_BYTES:
+        np.save(os.path.join(out_dir, 'H.npy'), be.to_ndarray(H))
+    else:
+        idx = np.sort(np.random.default_rng(0).choice(H.numel(), H_SAMPLE, replace=False))
+        np.save(os.path.join(out_dir, 'H_sample.npy'), be.to_ndarray(torch.take(H, torch.from_numpy(idx).to(H.device))))
+
+
 def run_b200(args, w):
     import torch
     import torch.distributed as dist
@@ -331,13 +373,15 @@ def run_b200(args, w):
     gen = torch.Generator(device=device)
     gen.manual_seed(1234 + rank)
     V = torch.rand((n_local, w['C'], *w['D']), dtype=torch.float32, device=device, generator=gen)
-    torch.manual_seed(99)       # same W on every rank (it is broadcast anyway)
+    torch.manual_seed(99)       # the start values the library draws itself in the e2e and cfg3 legs below (those of
+                                # the timed loop are replaced by seed_start_values)
 
     nmf = TransformInvariantNMF(n_atoms=w['M'], atom_shape=w['A'], backend='b200', init='device',
                                 input_is_local_shard=True, kernel_path=args.kernel_path,
                                 cuda_graph=not args.no_cuda_graph)
     be = nmf._backend                                                    # pylint: disable=protected-access
     nmf._initialize_matrices(V, keep_W=False)                            # pylint: disable=protected-access
+    seed_start_values(nmf, device, rank)
 
     # one batch MU iteration exactly as fit_batch runs it: eager the first time, CUDA-graph replays afterwards
     step = nmf._batch_step()                                             # pylint: disable=protected-access
@@ -367,6 +411,8 @@ def run_b200(args, w):
     t_wall1 = time.perf_counter()
     launches = be.launches - launches0
     clocks = sampler.stop(t_wall0, t_wall1) if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, be, nmf.W_device, nmf.H_device)
     # per-kernel durations: the same iteration launched eagerly with a CUDA-event pair around every hot-path call
     be.kernel_events = {}
     n_probe = min(args.steps, 5)
@@ -541,7 +587,9 @@ def finish_ranks(world, dist):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=50)
+    ap.add_argument('--steps', type=int, default=50,
+                    help='timed iterations of the headline loop and of the e2e leg; the cfg3 leg of a cfg2 run always '
+                         'times 5 (see measure_cfg3)')
     ap.add_argument('--warmup', type=int, default=3)
     ap.add_argument('--impl', default='b200', choices=['b200', 'reference'])
     ap.add_argument('--workload', default='cfg2', choices=sorted(WORKLOADS))
@@ -551,7 +599,13 @@ def main():
     ap.add_argument('--no-cfg3', action='store_true', help='skip the cfg3 strong-scaling leg of the cfg2 run')
     ap.add_argument('--samples', type=int, default=0, help='samples per GPU instead of the workload default '
                     '(e.g. --workload cfg5 --samples 512: BASELINE config 5 at its full batch)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write W and H after the last timed step as .npy files to DIR (own arm only)')
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs applies to --impl b200')
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     args.warmup = max(args.warmup, 3) if args.impl == 'b200' else args.warmup
     w = dict(WORKLOADS[args.workload])
     if args.samples > 0:
