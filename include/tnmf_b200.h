@@ -53,7 +53,10 @@ extern "C" {
                                * single-channel rank-1 batches, which run as one 2-D image of signal rows) */
 #define TNMF_PATH_TC      4   /* tcgen05 3xTF32 tensor-core kernels with TMEM accumulators (reconstruction, H gradient /
                                  update, W gradient: rank 2, float, valid/full, atom height <= 15, C * atom width <= 64;
-                                 reconstruction: C <= 4, atoms <= 64); operations / shapes without one use the TMA family */
+                                 reconstruction: C <= 4, atoms <= 64); operations / shapes without one use the TMA family.
+                                 Rank 3 (float, valid): the same kernels over (sample, z-plane) pairs - reconstruction
+                                 and W gradient one launch per atom plane, the H update with the atom planes as channels
+                                 (C * A_z * A_x <= 64); reconstruction C <= 2, W gradient C * A_x <= 16, generic otherwise */
 
 /* tnmf_problem.flags: switches of the 'auto' family choice (diagnostics / tests; 0 = the library's defaults).  They are part
  * of the problem description so that every behaviour of the library is reproducible through this interface alone. */

@@ -14,6 +14,10 @@ Two groups of methods:
   * fused entry points (`update_H`, `gradient_W`, `apply_W_update`, `energy`) used by
     `tnmf_b200.TransformInvariantNMF`, which fold the facade's multiplicative-update arithmetic
     (tnmf/TransformInvariantNMF.py:217-271) into the kernels' epilogues.
+
+Three shift axes (volumes, videos as (t, y, x)): float32 'valid' problems run the reconstruction, the H update and the W
+gradient on the tcgen05 kernels over (sample, z-plane) pairs wherever they plan (DESIGN.md §3.10); float64, 'full' and
+'circular' volumes, and shapes no tensor-core kernel plans for, run on the generic kernels.  'auto' picks the path.
 """
 import ctypes
 from contextlib import contextmanager

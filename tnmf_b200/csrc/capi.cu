@@ -113,6 +113,7 @@ bool tc_gradw_ns_worthwhile(const Geo &g) {
 // which of the three tensor-core W gradients serves a problem whose family is TNMF_PATH_TC
 enum { GRADW_NS = 0, GRADW_TS = 1, GRADW_SS = 2 };
 int tc_gradw_variant(const tnmf_problem *p, const Geo &g) {
+    if (plane_problem(g)) return GRADW_NS;
     const bool forced = p->path == TNMF_PATH_TC;
     if (tmem_operand_gradw_ns(g, p->dtype) && (forced || tc_gradw_ns_worthwhile(g))) return GRADW_NS;
     if (tmem_operand_gradw(g, p->dtype)) return GRADW_TS;
@@ -147,10 +148,30 @@ bool tc_recon_os_worthwhile(const Geo &g) {
 // which of the three tensor-core reconstructions serves a problem whose family is TNMF_PATH_TC
 enum { RECON_TS = 0, RECON_OS = 1, RECON_SS = 2 };
 int tc_recon_variant(const tnmf_problem *p, const Geo &g) {
+    if (plane_problem(g)) return RECON_OS;
     const bool forced = p->path == TNMF_PATH_TC;
     if (tmem_operand_recon(g, p->dtype) && (forced || tc_recon_ts_worthwhile(g))) return RECON_TS;
     if (tmem_operand_recon_os(g, p->dtype) && (forced || tc_recon_os_worthwhile(g))) return RECON_OS;
     return RECON_SS;
+}
+
+// 3-D problems (three shift axes in use) run on the plane mode of three tensor-memory kernels (DESIGN.md §3.10):
+// hupd_ts, recon_os (C <= 2) and gradw_ns (C * A_x <= 16), float32 'valid' only.  Their alternative is the generic
+// kernel, not the FP32 tiled / TMA ones (2-D only), so 'auto' takes them wherever they plan and at least half of every
+// 16-atom block is real atoms (a few atoms in a large padded MMA lose to nothing).  The TNMF_FLAG_NO_TC_* flags keep
+// 'auto' on the generic kernels, TNMF_FLAG_NO_TMEM_OPERAND keeps every path there.
+bool planes_tc(const tnmf_problem *p, const Geo &g, int op) {
+    if (g.flags & TNMF_FLAG_NO_TMEM_OPERAND) return false;
+    if (p->path == TNMF_PATH_AUTO) {
+        const int off = op == TNMF_OP_RECONSTRUCT ? TNMF_FLAG_NO_TC_RECON
+                      : op == TNMF_OP_GRADIENT_H  ? TNMF_FLAG_NO_TC_HUPD : TNMF_FLAG_NO_TC_GRADW;
+        if ((g.flags & off) || (double)g.M / ((g.M + 15) / 16 * 16) < 0.5) return false;
+    } else if (p->path != TNMF_PATH_TC) {
+        return false;
+    }
+    if (op == TNMF_OP_RECONSTRUCT) return tc_recon_os_supported(g, p->dtype);
+    if (op == TNMF_OP_GRADIENT_H) return tc_hupd_ts_supported(g, p->dtype);
+    return tc_gradw_ns_supported(g, p->dtype);
 }
 
 // Kernel family serving operation `op`: TMA where eligible, else the cp.async tiled kernels, else the generic ones;
@@ -158,6 +179,11 @@ int tc_recon_variant(const tnmf_problem *p, const Geo &g) {
 int choose_family(const tnmf_problem *p, const Geo &g, int op, int *err) {
     *err = TNMF_OK;
     if (p->path == TNMF_PATH_GENERIC) return TNMF_PATH_GENERIC;
+    if (plane_problem(g)) {                                     // (the tiled and TMA kernels are 2-D only)
+        if (planes_tc(p, g, op)) return TNMF_PATH_TC;
+        if (p->path == TNMF_PATH_TMA || p->path == TNMF_PATH_TILED) { *err = TNMF_EUNSUPPORTED; return -1; }
+        return TNMF_PATH_GENERIC;                                   // forced 'tc': tensor cores where a kernel plans
+    }
     if (op == TNMF_OP_GRADIENT_H && (p->path == TNMF_PATH_TC || (p->path == TNMF_PATH_AUTO && tc_worthwhile(g))) &&
         (tc_hupd_supported(g, p->dtype) || tmem_operand_hupd(g, p->dtype)))
         return TNMF_PATH_TC;
@@ -195,6 +221,10 @@ size_t align256(size_t b) { return (b + 255) & ~(size_t)255; }
 size_t energy_partials_bytes(const Geo &g) {
     return align256(sizeof(double) * (size_t)generic_energy_partial_capacity(g));
 }
+
+// the 3-D tensor-core reconstruction accumulates R over its per-plane launches: without a caller's R buffer it needs
+// R-sized scratch (behind the energy partials in the workspace)
+size_t r_scratch_bytes(const Geo &g) { return align256(sizeof(float) * (size_t)g.N * g.C * (size_t)vol3(g.D)); }
 
 }  // namespace
 
@@ -248,6 +278,10 @@ static size_t workspace_bytes_of(const Geo &g, int dtype) {
         const size_t w = align256(tc_gradw_ns_workspace_bytes(g));
         if (w > bytes) bytes = w;
     }
+    if (tc_recon_os_supported(g, dtype) && plane_problem(g)) {
+        const size_t w = energy_partials_bytes(g) + r_scratch_bytes(g);
+        if (w > bytes) bytes = w;
+    }
     return bytes;
 }
 
@@ -287,6 +321,8 @@ const char *tnmf_kernel_name(const tnmf_problem *p, int op) {
     if (f == TNMF_PATH_TILED) return names[op][1];
     if (f == TNMF_PATH_TMA) return names[op][2];
     if (f != TNMF_PATH_TC) return "none";
+    if (plane_problem(g))
+        return op == TNMF_OP_RECONSTRUCT ? "recon_os3_kernel" : op == TNMF_OP_GRADIENT_H ? "hupd_ts3_kernel" : "gradw_ns3_kernel";
     if (op == TNMF_OP_RECONSTRUCT) {
         const int v = tc_recon_variant(p, g);
         return v == RECON_TS ? "recon_ts_kernel" : v == RECON_OS ? "recon_os_kernel" : "recon_tc_kernel";
@@ -306,7 +342,7 @@ int tnmf_launch_count(const tnmf_problem *p, int op) {
     if (op == TNMF_OP_GRADIENT_W)                                                            // + the finishing reduction
         return f != TNMF_PATH_TC ? 2 : tc_gradw_variant(p, g) == GRADW_NS ? tc_gradw_ns_launches(g)
                                      : tc_gradw_variant(p, g) == GRADW_TS ? tc_gradw_ts_launches(g) : tc_gradw_launches(g);
-    if (f == TNMF_PATH_TC) return op == TNMF_OP_RECONSTRUCT ? 1 : tc_hupd_launches(g);
+    if (f == TNMF_PATH_TC) return op == TNMF_OP_RECONSTRUCT ? g.A[0] : tc_hupd_launches(g);    // (3-D: one per atom plane)
     return f == TNMF_PATH_TMA ? 2 : 1;                                                      // + the atom pre-arrangement
 }
 
@@ -369,6 +405,7 @@ int tnmf_reconstruct_energy(const tnmf_problem *p, const void *V, const void *W,
     if (family == TNMF_PATH_TC && tc_recon_variant(p, g) == RECON_TS) {
         s = tc_reconstruct_ts(g, (const float *)W, (const float *)H, (float *)R, (const float *)V, partials, &n_partials, st);
     } else if (family == TNMF_PATH_TC && tc_recon_variant(p, g) == RECON_OS) {
+        if (!R && plane_problem(g)) R = (char *)workspace + energy_partials_bytes(g);
         s = tc_reconstruct_os(g, (const float *)W, (const float *)H, (float *)R, (const float *)V, partials, &n_partials, st);
     } else if (family == TNMF_PATH_TC) {
         s = tc_reconstruct(g, (const float *)W, (const float *)H, (float *)R, (const float *)V, partials, &n_partials, st);

@@ -33,6 +33,9 @@ struct Geo {
 
 __host__ __device__ inline long long vol3(const int *s) { return (long long)s[0] * s[1] * s[2]; }
 
+// a third shift axis in use: the 2-D kernel families do not serve the problem (tc_common.cuh: plane mode)
+inline bool plane_problem(const Geo &g) { return g.D[0] != 1 || g.A[0] != 1; }
+
 // Map a logical index onto [0, extent): returns false when the element is an implicit zero.
 __device__ __forceinline__ bool fold_index(int &i, int extent, int wrap) {
     if (wrap) {

@@ -30,6 +30,44 @@ using tma::mbar_init;
 using tma::mbar_wait;
 using tma::smem_u32;
 
+// ---- plane mode: 3-D 'valid' problems on the 2-D tensor-memory kernels (DESIGN.md §3.10) ----------------------------
+// In 'valid' mode a 3-D correlation is a sum over the atom plane a_z of 2-D correlations between z-planes, so the 2-D
+// kernels run over VIRTUAL SAMPLES nv = n * NZ + z (one z-plane of sample n each) with a two-level address:
+//   V / R plane z of sample n, channel c:  n * xsn + c * xsc + z * D_y * D_x
+//   H plane t of sample n, atom m:         n * hsn + m * hsm + t * hsz
+// The reconstruction and the W gradient launch once per a_z (NZ = D_z, H shifted by offz - az planes); the H update
+// launches once, its a_z planes being extra channels (c, a_z) of the contraction (NZ = T_z, Geo2::C = C * A_z).
+struct Geo3 : tiled::Geo2 {
+    int NZ;                 // planes per sample in the virtual sample index
+    int DZ, AZ, offz;       // sample planes, atom planes, A_z - 1
+    int az;                 // atom plane of this launch (reconstruction, W gradient)
+    int acc;                // reconstruction: add to R instead of writing it (every launch after the first)
+    long long xsn, xsc;     // element strides of V / R between samples and between channels
+    long long hsz;          // element stride between activation planes (T_y * hsy)
+};
+
+// 3-D problems the plane mode serves: float32 'valid' (off = A - 1 on every axis)
+inline bool plane_mode_ok(const Geo &g, int dtype) {
+    if (dtype != TNMF_F32 || g.wrap || !plane_problem(g) || g.N < 1) return false;
+    for (int i = 0; i < 3; ++i)
+        if (g.off[i] != g.A[i] - 1 || g.T[i] != g.D[i] + g.A[i] - 1) return false;
+    return true;
+}
+// h_update: virtual samples over the activation planes, virtual channels (c, a_z); otherwise over the sample planes
+inline Geo3 make_geo3(const Geo &g, bool h_update, int az = 0) {
+    Geo3 q;
+    static_cast<tiled::Geo2 &>(q) = tiled::make_geo2(g);
+    q.NZ = h_update ? g.T[0] : g.D[0];
+    q.N = g.N * q.NZ;
+    if (h_update) q.C = g.C * g.A[0];
+    q.DZ = g.D[0]; q.AZ = g.A[0]; q.offz = g.off[0];
+    q.az = az; q.acc = 0;
+    q.xsc = (long long)g.D[0] * g.D[1] * g.D[2];
+    q.xsn = q.xsc * g.C;
+    q.hsz = (long long)g.T[1] * g.hsy;
+    return q;
+}
+
 // Wait with back-off for roles that are far from the critical path: every poll of a spinning warp is a shared-memory
 // wavefront, and shared-memory bandwidth is what bounds the tensor-core kernels (ncu: polls were 30% of the LSU traffic).
 __device__ __forceinline__ void mbar_wait_backoff(unsigned long long *bar, unsigned parity, unsigned ns) {

@@ -131,7 +131,10 @@ __device__ __forceinline__ Unit make_unit(long long u, const Geo2 &g, const Plan
     return w;
 }
 
-__global__ void __launch_bounds__(kThreads, 1) gradw_ns_kernel(const Geo2 g, const Plan p, const Args a) {
+// P3: plane mode (G = Geo3, tc_common.cuh) - virtual samples (n, z), H shifted by the host to plane z + offz - az, the
+// partial slices indexed [m][c][a_z][a_y][a_x] with this launch's a_z
+template <bool P3, class G>
+__device__ __forceinline__ void gradw_ns_body(const G &g, const Plan &p, const Args &a) {
     extern __shared__ __align__(128) float smem[];
     __shared__ __align__(8) unsigned long long a_full[kMaxAStages], a_empty[kMaxAStages], h_full[kRingMax / 2], h_free[kRingMax / 2],
         set_done[2], set_free[2];
@@ -162,7 +165,8 @@ __global__ void __launch_bounds__(kThreads, 1) gradw_ns_kernel(const Geo2 g, con
     __syncthreads();
     tc_fence_after();
 
-    const long long count = (long long)g.M * C * AY * AX;
+    long long count = (long long)g.M * C * AY * AX;
+    if constexpr (P3) count *= g.AZ;
 
     if (warp < 8) {
         // ------------------------------------ workers ------------------------------------
@@ -206,7 +210,10 @@ __global__ void __launch_bounds__(kThreads, 1) gradw_ns_kernel(const Geo2 g, con
                     const long long J = (long long)w.tile * kCT + xr;
                     const int n = (int)(J / p.TXP);
                     const int x = (int)(J - (long long)n * p.TXP) - g.offx;
-                    if (n < g.N && (unsigned)x < (unsigned)g.DX) roff[e] = ((long long)n * C + c) * plane + x;
+                    if (n < g.N && (unsigned)x < (unsigned)g.DX) {
+                        if constexpr (P3) roff[e] = (n / g.NZ) * g.xsn + c * g.xsc + (long long)(n % g.NZ) * plane + x;
+                        else roff[e] = ((long long)n * C + c) * plane + x;
+                    }
                 }
             }
             long long hoff[4];
@@ -215,8 +222,10 @@ __global__ void __launch_bounds__(kThreads, 1) gradw_ns_kernel(const Geo2 g, con
                 const long long J = (long long)w.tile * kCT + 4 * h_cg + e;
                 const int n = (int)(J / p.TXP);
                 const int xv = (int)(J - (long long)n * p.TXP);
-                hoff[e] = (n < g.N && xv < g.TX && a.m0 + h_ml < g.M)
-                              ? (long long)n * g.hsn + (long long)(a.m0 + h_ml) * g.hsm + xv : -1;
+                long long hbase;
+                if constexpr (P3) hbase = (long long)(n / g.NZ) * g.hsn + (long long)(n % g.NZ) * g.hsz;
+                else hbase = (long long)n * g.hsn;
+                hoff[e] = (n < g.N && xv < g.TX && a.m0 + h_ml < g.M) ? hbase + (long long)(a.m0 + h_ml) * g.hsm + xv : -1;
             }
             auto load_raw = [&](int r, float (&rv)[kRawMax]) {
 #pragma unroll
@@ -338,8 +347,12 @@ __global__ void __launch_bounds__(kThreads, 1) gradw_ns_kernel(const Geo2 g, con
         const bool live = k < p.KPL;
         const int c = live ? k / AX : 0, ax = live ? k - c * AX : 0;
         float *slice = a.partials + ((long long)blockIdx.x * 4 + part * 2 + s_l) * 2 * count + (long long)X_l * count;
-        const long long mstride = (long long)C * AY * AX;
+        long long mstride = (long long)C * AY * AX;
         float *dst_base = slice + (((long long)a.m0 * C + c) * AY) * AX + ax;
+        if constexpr (P3) {
+            mstride *= g.AZ;
+            dst_base = slice + ((((long long)a.m0 * C + c) * g.AZ + g.az) * AY) * AX + ax;
+        }
         TC_PROF_DECL(done); TC_PROF_DECL(total);
 #ifdef TNMF_TC_PROFILE
         prof_total = -clock64();
@@ -461,45 +474,65 @@ __global__ void __launch_bounds__(kThreads, 1) gradw_ns_kernel(const Geo2 g, con
     if (warp == 8) tmem_dealloc(tmem_base, 512);
 }
 
+__global__ void __launch_bounds__(kThreads, 1) gradw_ns_kernel(const Geo2 g, const Plan p, const Args a) {
+    gradw_ns_body<false>(g, p, a);
+}
+__global__ void __launch_bounds__(kThreads, 1) gradw_ns3_kernel(const Geo3 g, const Plan p, const Args a) {
+    gradw_ns_body<true>(g, p, a);
+}
+
 }  // namespace gwn
 }  // namespace tc
 
 // ---- dispatch ----------------------------------------------------------------------------------------------------------
 bool tc_gradw_ns_supported(const Geo &g, int dtype) {
+    tc::gwn::Plan p;
+    if (plane_problem(g)) return tc::plane_mode_ok(g, dtype) && tc::gwn::make_plan(tc::make_geo3(g, false), p);
     if (dtype != TNMF_F32 || g.wrap) return false;
     if (g.D[0] != 1 || g.A[0] != 1 || g.T[0] != 1) return false;      // rank <= 2
     if (g.D[1] == 1 && g.A[1] == 1) return false;                     // rank 1: the FP32 kernels serve it
     if (g.N < 1) return false;
-    tc::gwn::Plan p;
     return tc::gwn::make_plan(tiled::make_geo2(g), p);
 }
 
 size_t tc_gradw_ns_workspace_bytes(const Geo &g) {
     tc::gwn::Plan p;
-    if (!tc::gwn::make_plan(tiled::make_geo2(g), p)) return 0;
-    return (size_t)p.grid * 4 * 2 * (size_t)g.M * g.C * g.A[1] * g.A[2] * sizeof(float);
+    const bool planes = plane_problem(g);
+    if (!(planes ? tc::gwn::make_plan(tc::make_geo3(g, false), p) : tc::gwn::make_plan(tiled::make_geo2(g), p))) return 0;
+    return (size_t)p.grid * 4 * 2 * (size_t)g.M * g.C * (size_t)vol3(g.A) * sizeof(float);
 }
 
 int tc_gradient_w_ns(const Geo &g, const float *V, const float *R, const float *H, float *neg, float *pos, void *workspace,
                      size_t workspace_bytes, cudaStream_t st) {
-    const tiled::Geo2 q = tiled::make_geo2(g);
+    const bool planes = plane_problem(g);
+    tc::Geo3 q3 = tc::make_geo3(g, false);
+    const tiled::Geo2 q = planes ? q3 : tiled::make_geo2(g);
     tc::gwn::Plan p;
     if (!tc::gwn::make_plan(q, p)) return TNMF_EUNSUPPORTED;
-    const long long count = (long long)g.M * g.C * g.A[1] * g.A[2];
+    const long long count = (long long)g.M * g.C * vol3(g.A);
     if (!workspace || workspace_bytes < tc_gradw_ns_workspace_bytes(g)) return TNMF_EWORKSPACE;
     tc::gwn::Args a;
     a.V = V; a.R = R; a.H = H; a.partials = (float *)workspace;
     auto kern = tc::gwn::gradw_ns_kernel;
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::gwn::kMaxSmem);
+    auto kern3 = tc::gwn::gradw_ns3_kernel;
+    cudaError_t e = cudaFuncSetAttribute(planes ? (const void *)kern3 : (const void *)kern,
+                                         cudaFuncAttributeMaxDynamicSharedMemorySize, tc::gwn::kMaxSmem);
     if (e != cudaSuccess) return status_from_cuda(e);
-    for (int m0 = 0; m0 < g.M; m0 += tc::gwn::kNB) {
-        a.m0 = m0;
-        kern<<<(unsigned)p.grid, tc::gwn::kThreads, p.smem, st>>>(q, p, a);
-        TNMF_CHECK_LAUNCH();
+    // 3-D: one pass per atom plane a_z over the virtual samples (n, z), against H shifted by offz - a_z planes; each pass
+    // fills its own a_z slice of every partial, and one fixed-order reduction finishes all of them
+    for (int az = 0; az < (planes ? g.A[0] : 1); ++az) {
+        q3.az = az;
+        a.H = planes ? H + (long long)(q3.offz - az) * q3.hsz : H;
+        for (int m0 = 0; m0 < g.M; m0 += tc::gwn::kNB) {
+            a.m0 = m0;
+            if (planes) kern3<<<(unsigned)p.grid, tc::gwn::kThreads, p.smem, st>>>(q3, p, a);
+            else kern<<<(unsigned)p.grid, tc::gwn::kThreads, p.smem, st>>>(q, p, a);
+            TNMF_CHECK_LAUNCH();
+        }
     }
     return finish_gradient_w<float>((const float *)workspace, p.grid * 4, count, neg, pos, st);
 }
 
-int tc_gradw_ns_launches(const Geo &g) { return tiled::ceil_div(g.M, tc::gwn::kNB) + 1; }
+int tc_gradw_ns_launches(const Geo &g) { return g.A[0] * tiled::ceil_div(g.M, tc::gwn::kNB) + 1; }
 
 }  // namespace tnmf

@@ -126,9 +126,11 @@ __device__ __forceinline__ Unit make_unit(long long u, const Geo2 &g, const Plan
     return w;
 }
 
-// KPT = KP: compile-time contraction length (the expansion is fully unrolled: all loads of a row in flight at once)
-template <int KPT>
-__global__ void __launch_bounds__(kThreads, 1) hupd_ts_kernel(const Geo2 g, const Plan p, const Args a) {
+// KPT = KP: compile-time contraction length (the expansion is fully unrolled: all loads of a row in flight at once);
+// P3: plane mode (G = Geo3, tc_common.cuh) - virtual samples (n, t_z), virtual channels (c, a_z) reading source plane
+// t_z - offz + a_z, or zeros outside [0, D_z)
+template <int KPT, bool P3, class G>
+__device__ __forceinline__ void hupd_ts_body(const G &g, const Plan &p, const Args &a) {
     extern __shared__ __align__(128) float smem[];
     __shared__ __align__(8) unsigned long long a_full[2], a_empty[2], turn[2], x_done[2][kRingMax], x_free[2][kRingMax];
     __shared__ unsigned tmem_base_s;
@@ -204,7 +206,14 @@ __global__ void __launch_bounds__(kThreads, 1) hupd_ts_kernel(const Geo2 g, cons
                     const long long J = (long long)w.tile * kTile + (q - c * RW);
                     const int n = (int)(J / p.TXP);
                     const int x = (int)(J - (long long)n * p.TXP) - g.offx;
-                    if (n < g.N && (unsigned)x < (unsigned)g.DX) roff[e] = ((long long)n * C + c) * plane + x;
+                    if (n < g.N && (unsigned)x < (unsigned)g.DX) {
+                        if constexpr (P3) {
+                            const int ns = n / g.NZ, cr = c / g.AZ, z = n - ns * g.NZ - g.offz + (c - cr * g.AZ);
+                            if ((unsigned)z < (unsigned)g.DZ) roff[e] = ns * g.xsn + cr * g.xsc + (long long)z * plane + x;
+                        } else {
+                            roff[e] = ((long long)n * C + c) * plane + x;
+                        }
+                    }
                 }
             }
             float rv[kRawMax];
@@ -294,7 +303,10 @@ __global__ void __launch_bounds__(kThreads, 1) hupd_ts_kernel(const Geo2 g, cons
             const bool active = n < g.N && tx < g.TX;
             // the activations of a row do not depend on the accumulators: they are fetched one row ahead
             float hnext[kHA];
-            float *hrow = (a.H && active) ? a.H + (long long)n * g.hsn + (long long)ma * g.hsm + tx : nullptr;
+            long long hbase;
+            if constexpr (P3) hbase = (long long)(n / g.NZ) * g.hsn + (long long)(n % g.NZ) * g.hsz;
+            else hbase = (long long)n * g.hsn;
+            float *hrow = (a.H && active) ? a.H + hbase + (long long)ma * g.hsm + tx : nullptr;
             auto load_h = [&](int ty) {
 #pragma unroll
                 for (int ml = 0; ml < kHA; ++ml)
@@ -353,7 +365,9 @@ __global__ void __launch_bounds__(kThreads, 1) hupd_ts_kernel(const Geo2 g, cons
                 for (int ml = 0; ml < kHA; ++ml) {
                     const int m = ma + ml;
                     if (m >= g.M) continue;
-                    const long long cidx = ((long long)n * g.M + m) * tvol + tin;
+                    long long cidx;                 // dense [n][m][(t_z,) t_y][t_x]; Gsum has one atom: n * tvol suits both
+                    if constexpr (P3) cidx = (((long long)(n / g.NZ) * g.M + m) * g.NZ + n % g.NZ) * tvol + tin;
+                    else cidx = ((long long)n * g.M + m) * tvol + tin;
                     if (a.H) {
                         const float h = hv[ml];
                         float ps = pos[ml];
@@ -482,8 +496,20 @@ __global__ void __launch_bounds__(kThreads, 1) hupd_ts_kernel(const Geo2 g, cons
 }
 
 template <int KPT>
-static int launch(const Geo2 &g, const Plan &p, const Args &a, cudaStream_t st) {
-    auto kern = hupd_ts_kernel<KPT>;
+__global__ void __launch_bounds__(kThreads, 1) hupd_ts_kernel(const Geo2 g, const Plan p, const Args a) {
+    hupd_ts_body<KPT, false>(g, p, a);
+}
+template <int KPT>
+__global__ void __launch_bounds__(kThreads, 1) hupd_ts3_kernel(const Geo3 g, const Plan p, const Args a) {
+    hupd_ts_body<KPT, true>(g, p, a);
+}
+
+template <int KPT> static auto kernel_for(const Geo2 &) { return hupd_ts_kernel<KPT>; }
+template <int KPT> static auto kernel_for(const Geo3 &) { return hupd_ts3_kernel<KPT>; }
+
+template <int KPT, class G>
+static int launch(const G &g, const Plan &p, const Args &a, cudaStream_t st) {
+    auto kern = kernel_for<KPT>(g);
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxSmem);
     if (e != cudaSuccess) return status_from_cuda(e);
     kern<<<(unsigned)p.grid, kThreads, p.smem, st>>>(g, p, a);
@@ -496,24 +522,26 @@ static int launch(const Geo2 &g, const Plan &p, const Args &a, cudaStream_t st) 
 
 // ---- dispatch ----------------------------------------------------------------------------------------------------------
 bool tc_hupd_ts_supported(const Geo &g, int dtype) {
+    tc::hut::Plan p;
+    if (plane_problem(g)) return tc::plane_mode_ok(g, dtype) && tc::hut::make_plan(tc::make_geo3(g, true), p);
     if (dtype != TNMF_F32 || g.wrap) return false;
     if (g.D[0] != 1 || g.A[0] != 1 || g.T[0] != 1) return false;      // rank <= 2
     if (g.D[1] == 1 && g.A[1] == 1) return false;                     // rank 1: the FP32 kernels serve it
     if (g.N < 1) return false;
-    tc::hut::Plan p;
     return tc::hut::make_plan(tiled::make_geo2(g), p);
 }
 
-int tc_gradient_h_ts(const Geo &g, const float *V, const float *R, const float *W, float *neg, float *pos, float *H,
-                     double reg, const float *G, double lambda, const float *Gsum, double lambda_cross, cudaStream_t st) {
-    const tiled::Geo2 q = tiled::make_geo2(g);
+template <class G>
+static int gradient_h_ts(const G &q, int M, const float *V, const float *R, const float *W, float *neg, float *pos,
+                         float *H, double reg, const float *G_, double lambda, const float *Gsum, double lambda_cross,
+                         cudaStream_t st) {
     tc::hut::Plan p;
     if (!tc::hut::make_plan(q, p)) return TNMF_EUNSUPPORTED;
     tc::hut::Args a;
     a.V = V; a.R = R; a.W = W; a.neg = neg; a.pos = pos; a.H = H;
     a.reg = (float)reg; a.lambda = (float)lambda; a.lambda_cross = (float)lambda_cross;
-    a.G = G; a.Gsum = Gsum;
-    for (int m0 = 0; m0 < g.M; m0 += tc::hut::kNB) {
+    a.G = G_; a.Gsum = Gsum;
+    for (int m0 = 0; m0 < M; m0 += tc::hut::kNB) {
         a.m0 = m0;
         int s;
         switch (p.KP) {
@@ -530,6 +558,15 @@ int tc_gradient_h_ts(const Geo &g, const float *V, const float *R, const float *
         if (s) return s;
     }
     return TNMF_OK;
+}
+
+int tc_gradient_h_ts(const Geo &g, const float *V, const float *R, const float *W, float *neg, float *pos, float *H,
+                     double reg, const float *G, double lambda, const float *Gsum, double lambda_cross, cudaStream_t st) {
+    // 3-D: ONE launch per block of atoms - the a_z planes are channels of the contraction, so the fused epilogue sees
+    // complete sums
+    if (plane_problem(g))
+        return gradient_h_ts(tc::make_geo3(g, true), g.M, V, R, W, neg, pos, H, reg, G, lambda, Gsum, lambda_cross, st);
+    return gradient_h_ts(tiled::make_geo2(g), g.M, V, R, W, neg, pos, H, reg, G, lambda, Gsum, lambda_cross, st);
 }
 
 }  // namespace tnmf

@@ -127,9 +127,11 @@ __device__ __forceinline__ void tmem_st4(unsigned addr, float a, float b, float 
                  : "memory");
 }
 
-// C: channels (compile time: the epilogue's sums live in registers); APT: atoms per stage-writing thread = KM / 2
-template <int C, int APT>
-__global__ void __launch_bounds__(kThreads, 1) recon_os_kernel(const Geo2 g, const Plan p, const Args a) {
+// C: channels (compile time: the epilogue's sums live in registers); APT: atoms per stage-writing thread = KM / 2;
+// P3: plane mode (G = Geo3, tc_common.cuh) - virtual samples (n, z), H shifted by the host to plane z + offz - az, atom
+// plane az of W, and R accumulated over the launches of one reconstruction (g.acc)
+template <int C, int APT, bool P3, class G>
+__device__ __forceinline__ void recon_os_body(const G &g, const Plan &p, const Args &a) {
     extern __shared__ __align__(128) float smem[];
     __shared__ __align__(8) unsigned long long a_full[kStageMax], a_free[kStageMax], d_full[kRingMax], d_free[kRingMax];
     __shared__ unsigned tmem_base_s;
@@ -151,7 +153,8 @@ __global__ void __launch_bounds__(kThreads, 1) recon_os_kernel(const Geo2 g, con
         float v = 0.f;
         if (r < NU && m < g.M) {
             const int c = r / AX, ax = r - c * AX;
-            v = a.W[(((long long)m * C + c) * AY + ay) * AX + ax];
+            if constexpr (P3) v = a.W[((((long long)m * C + c) * g.AZ + g.az) * AY + ay) * AX + ax];
+            else v = a.W[(((long long)m * C + c) * AY + ay) * AX + ax];
         }
         float hi, lo;
         split_tf32(v, hi, lo);
@@ -193,7 +196,10 @@ __global__ void __launch_bounds__(kThreads, 1) recon_os_kernel(const Geo2 g, con
             const int v = (int)(F - (long long)n * p.VW) + g.offx - (AX - 1);
             const bool real = n < g.N && (unsigned)v < (unsigned)g.TX;
             // two rows are always in flight (the activations come from DRAM: ~1000 clk against ~1500 clk per row)
-            const float *hnext = a.H + (real ? (long long)n * g.hsn + (long long)m_lo * g.hsm + v + (long long)w.ta * g.hsy : 0);
+            long long hbase;
+            if constexpr (P3) hbase = (long long)(n / g.NZ) * g.hsn + (long long)(n % g.NZ) * g.hsz;
+            else hbase = (long long)n * g.hsn;
+            const float *hnext = a.H + (real ? hbase + (long long)m_lo * g.hsm + v + (long long)w.ta * g.hsy : 0);
             const int mv = real ? m_valid : 0;
             float hva[APT], hvb[APT];
             auto load_row = [&](float (&hv)[APT]) {
@@ -255,7 +261,13 @@ __global__ void __launch_bounds__(kThreads, 1) recon_os_kernel(const Geo2 g, con
             const int n = (int)(F0 / p.VW);
             const int xo = (int)(F0 - (long long)n * p.VW);
             const bool active = i < p.S && n < g.N && xo < g.DX;
-            const long long obase = (long long)n * C * plane + xo;
+            long long obase, cstride = plane;
+            if constexpr (P3) {
+                obase = (long long)(n / g.NZ) * g.xsn + (long long)(n % g.NZ) * plane + xo;
+                cstride = g.xsc;
+            } else {
+                obase = (long long)n * C * plane + xo;
+            }
             for (int y = w.y0; y < w.y1; ++y, ++row) {
                 const int my_slot = slot;
                 const unsigned my_par = slot_wraps & 1u;
@@ -316,7 +328,10 @@ __global__ void __launch_bounds__(kThreads, 1) recon_os_kernel(const Geo2 g, con
                     }
 #pragma unroll
                     for (int c = 0; c < C; ++c) {
-                        const long long o = obase + (long long)c * plane + (long long)y * g.DX;
+                        const long long o = obase + (long long)c * cstride + (long long)y * g.DX;
+                        if constexpr (P3) {
+                            if (g.acc) r[c] = a.R[o] + r[c];
+                        }
                         if (a.R) a.R[o] = r[c];
                         if (a.V) {
                             const double d = (double)a.V[o] - (double)r[c];
@@ -472,8 +487,19 @@ __global__ void __launch_bounds__(kThreads, 1) recon_os_kernel(const Geo2 g, con
 }
 
 template <int C, int APT>
-static int launch2(const Geo2 &g, const Plan &p, const Args &a, cudaStream_t st) {
-    auto kern = recon_os_kernel<C, APT>;
+__global__ void __launch_bounds__(kThreads, 1) recon_os_kernel(const Geo2 g, const Plan p, const Args a) {
+    recon_os_body<C, APT, false>(g, p, a);
+}
+template <int C, int APT>
+__global__ void __launch_bounds__(kThreads, 1) recon_os3_kernel(const Geo3 g, const Plan p, const Args a) {
+    recon_os_body<C, APT, true>(g, p, a);
+}
+template <int C, int APT> static auto kernel_for(const Geo2 &) { return recon_os_kernel<C, APT>; }
+template <int C, int APT> static auto kernel_for(const Geo3 &) { return recon_os3_kernel<C, APT>; }
+
+template <int C, int APT, class G>
+static int launch2(const G &g, const Plan &p, const Args &a, cudaStream_t st) {
+    auto kern = kernel_for<C, APT>(g);
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kMaxSmem);
     if (e != cudaSuccess) return status_from_cuda(e);
     kern<<<(unsigned)p.grid, kThreads, p.smem, st>>>(g, p, a);
@@ -481,8 +507,8 @@ static int launch2(const Geo2 &g, const Plan &p, const Args &a, cudaStream_t st)
     return TNMF_OK;
 }
 
-template <int C>
-static int launch(const Geo2 &g, const Plan &p, const Args &a, cudaStream_t st) {
+template <int C, class G>
+static int launch(const G &g, const Plan &p, const Args &a, cudaStream_t st) {
     switch (p.KM / 2) {
         case 4: return launch2<C, 4>(g, p, a, st);
         case 8: return launch2<C, 8>(g, p, a, st);
@@ -497,32 +523,56 @@ static int launch(const Geo2 &g, const Plan &p, const Args &a, cudaStream_t st) 
 
 // ---- dispatch ----------------------------------------------------------------------------------------------------------
 bool tc_recon_os_supported(const Geo &g, int dtype) {
+    tc::rco::Plan p;
+    if (plane_problem(g))
+        return g.C <= 2 && tc::plane_mode_ok(g, dtype) && tc::rco::make_plan(tc::make_geo3(g, false), p);
     if (dtype != TNMF_F32 || g.wrap) return false;
     if (g.D[0] != 1 || g.A[0] != 1 || g.T[0] != 1) return false;      // rank <= 2
     if (g.D[1] == 1 && g.A[1] == 1) return false;                     // rank 1: the FP32 kernels serve it
     if (g.N < 1 || g.C > 2) return false;
-    tc::rco::Plan p;
     return tc::rco::make_plan(tiled::make_geo2(g), p);
 }
 
 int tc_recon_os_partials(const Geo &g) {
     tc::rco::Plan p;
-    return tc::rco::make_plan(tiled::make_geo2(g), p) ? p.grid * 4 * tc::rco::kEpiGroups : 0;
+    const bool ok = plane_problem(g) ? tc::rco::make_plan(tc::make_geo3(g, false), p)
+                                         : tc::rco::make_plan(tiled::make_geo2(g), p);
+    return ok ? p.grid * 4 * tc::rco::kEpiGroups : 0;
 }
 
-int tc_reconstruct_os(const Geo &g, const float *W, const float *H, float *R, const float *V, double *energy_partials,
-                      int *n_partials, cudaStream_t st) {
-    const tiled::Geo2 q = tiled::make_geo2(g);
-    tc::rco::Plan p;
-    if (!tc::rco::make_plan(q, p)) return TNMF_EUNSUPPORTED;
-    tc::rco::Args a;
-    a.W = W; a.H = H; a.V = V; a.R = R; a.epart = energy_partials;
-    if (n_partials) *n_partials = p.grid * 4 * tc::rco::kEpiGroups;
+template <class G>
+static int reconstruct_os(const G &q, const Geo &g, const tc::rco::Plan &p, const tc::rco::Args &a, cudaStream_t st) {
     switch (g.C) {
         case 1: return tc::rco::launch<1>(q, p, a, st);
         case 2: return tc::rco::launch<2>(q, p, a, st);
         default: return TNMF_EUNSUPPORTED;
     }
+}
+
+int tc_reconstruct_os(const Geo &g, const float *W, const float *H, float *R, const float *V, double *energy_partials,
+                      int *n_partials, cudaStream_t st) {
+    const bool planes = plane_problem(g);
+    tc::Geo3 q3 = tc::make_geo3(g, false);
+    const tiled::Geo2 q = planes ? q3 : tiled::make_geo2(g);
+    tc::rco::Plan p;
+    if (!tc::rco::make_plan(q, p)) return TNMF_EUNSUPPORTED;
+    tc::rco::Args a;
+    a.W = W; a.H = H; a.V = V; a.R = R; a.epart = energy_partials;
+    if (n_partials) *n_partials = p.grid * 4 * tc::rco::kEpiGroups;
+    if (!planes) return reconstruct_os(q, g, p, a, st);
+    // 3-D: one launch per atom plane a_z, in order - the first writes R, the others add to it (deterministic); the last
+    // one holds the complete R and computes the energy partials
+    if (!R) return TNMF_EINVAL;
+    for (int az = 0; az < g.A[0]; ++az) {
+        q3.az = az;
+        q3.acc = az > 0;
+        a.H = H + (long long)(q3.offz - az) * q3.hsz;
+        a.V = az + 1 == g.A[0] ? V : nullptr;
+        a.epart = az + 1 == g.A[0] ? energy_partials : nullptr;
+        const int s = reconstruct_os(q3, g, p, a, st);
+        if (s) return s;
+    }
+    return TNMF_OK;
 }
 
 }  // namespace tnmf
