@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define TNMF_ABI_VERSION 5
+#define TNMF_ABI_VERSION 6
 #define TNMF_MAX_SHIFT_DIMS 3
 
 /* element types */
@@ -163,6 +163,24 @@ int tnmf_update_h(const tnmf_problem *p, const void *V, const void *R, const voi
  * Replaces Backend.reconstruction_gradient_W, tnmf/backends/_Backend.py:100-108 (NumPy.py:69-91). */
 int tnmf_gradient_w(const tnmf_problem *p, const void *V, const void *R, const void *H,
                     void *neg, void *pos, void *workspace, size_t workspace_bytes, void *stream);
+
+/* Plane windows: tnmf_update_h / tnmf_gradient_w restricted to the activation indices t in [t_lo, t_hi) along the FIRST
+ * shift axis (z-planes of a volume, rows of an image, positions of a signal).  The H update writes H only inside the
+ * window (it reads H, V and R wherever the correlations need them); the W gradient sums over the window only, as if H
+ * were zero outside it.  A band of a halo-sharded fit (tnmf_b200/halo.py) uses them to skip its halo planes, which the
+ * next exchange overwrites and which belong to the neighbours' share of the W gradient.  0 <= t_lo <= t_hi <= T[0] (else
+ * TNMF_EINVAL); the full window [0, T[0]) gives results bitwise equal to the unwindowed calls.
+ * Served by the plane mode of the tensor-core kernels (three shift axes, float32, 'valid') and by the generic kernels
+ * (any rank, mode and dtype); problems that another family serves return TNMF_EUNSUPPORTED.  tnmf_kernel_family and
+ * tnmf_kernel_name of the problem name the kernels a windowed call runs; tnmf_workspace_bytes and tnmf_launch_count of
+ * the problem bound what it needs and launches (the W gradient skips the per-atom-plane launches whose sample planes
+ * all lie outside the window). */
+int tnmf_update_h_planes(const tnmf_problem *p, const void *V, const void *R, const void *W, void *H,
+                         double reg, const void *G, double lambda, const void *Gsum, double lambda_cross,
+                         int32_t t_lo, int32_t t_hi, void *workspace, size_t workspace_bytes, void *stream);
+int tnmf_gradient_w_planes(const tnmf_problem *p, const void *V, const void *R, const void *H,
+                           void *neg, void *pos, int32_t t_lo, int32_t t_hi,
+                           void *workspace, size_t workspace_bytes, void *stream);
 
 /* W = (W * neg) / (pos + eps);  W[m,c,:] /= sum_a W[m,c,a].  In place; neg/pos are left untouched.
  * Replaces TransformInvariantNMF._update_W's arithmetic, tnmf/TransformInvariantNMF.py:217-244, and

@@ -30,7 +30,7 @@ MODES = {'valid': 0, 'full': 1, 'circular': 2}
 PATHS = {'auto': 0, 'generic': 1, 'tiled': 2, 'tma': 3, 'tc': 4}
 OP_RECONSTRUCT, OP_GRADIENT_H, OP_GRADIENT_W = 0, 1, 2
 TNMF_OK, TNMF_EINVAL, TNMF_EUNSUPPORTED, TNMF_EWORKSPACE, TNMF_ECUDA = 0, 1, 2, 3, 1000
-ABI_VERSION = 5
+ABI_VERSION = 6
 # tnmf_problem.flags (include/tnmf_b200.h)
 FLAG_NO_ROWS_VIEW, FLAG_ROWS_VIEW_ALWAYS = 1, 2
 FLAG_NO_TC_HUPD, FLAG_NO_TC_RECON, FLAG_NO_TC_GRADW, FLAG_NO_TC, FLAG_NO_TMA, FLAG_NO_TMEM_OPERAND = 4, 8, 16, 28, 32, 64
@@ -74,6 +74,8 @@ SIGNATURES = {
     'tnmf_gradient_h': (ctypes.c_int, [_P, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     'tnmf_update_h': (ctypes.c_int, [_P, _vp, _vp, _vp, _vp, _dbl, _vp, _dbl, _vp, _dbl, _vp, _sz, _vp]),
     'tnmf_gradient_w': (ctypes.c_int, [_P, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
+    'tnmf_update_h_planes': (ctypes.c_int, [_P, _vp, _vp, _vp, _vp, _dbl, _vp, _dbl, _vp, _dbl, _i32, _i32, _vp, _sz, _vp]),
+    'tnmf_gradient_w_planes': (ctypes.c_int, [_P, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _vp, _sz, _vp]),
     'tnmf_update_w': (ctypes.c_int, [_P, _vp, _vp, _vp, _dbl, _vp]),
     'tnmf_peer_buffer_bytes': (_sz, [_P, _i32]),
     'tnmf_allreduce_update_w': (ctypes.c_int, [_P, _vp, _vp, ctypes.POINTER(PeerWorld), _vp, _dbl, _vp]),

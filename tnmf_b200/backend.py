@@ -527,9 +527,12 @@ class B200_Backend(Backend):  # pylint: disable=invalid-name
 
     def update_H(self, V, W, H, s: slice = sliceNone, sparsity: float = 0., inhibition: float = 0.,
                  cross_inhibition: float = 0., inhibition_kernels: Optional[Sequence[np.ndarray]] = None,
-                 eps: float = 1.e-9, reuse_R: bool = False) -> None:
+                 eps: float = 1.e-9, reuse_R: bool = False, planes: Optional[Tuple[int, int]] = None) -> None:
         """One in-place multiplicative update of H[s]: reconstruct, both correlations, sparsity / inhibition terms and
-        H <- (H*neg)/pos in one fused kernel   (tnmf/TransformInvariantNMF.py:246-271 + :217-235)."""
+        H <- (H*neg)/pos in one fused kernel   (tnmf/TransformInvariantNMF.py:246-271 + :217-235).
+        `planes=(t_lo, t_hi)` updates only those activation indices along the first shift axis (tnmf_update_h_planes:
+        three shift axes, or any problem on the generic kernels); the reconstruction and the inhibition terms still see
+        all of H."""
         Hs = H[s]
         if Hs.shape[0] == 0:
             return
@@ -570,15 +573,24 @@ class B200_Backend(Backend):  # pylint: disable=invalid-name
         reg = eps + sparsity if sparsity > 0 else eps
         ws, ws_bytes = self._workspace(p)
         with self._timed('update_h'):
-            _lib.check(self._lib.tnmf_update_h(ctypes.byref(p), Vs.data_ptr(), R.data_ptr(), W.data_ptr(),
-                                               Hs.data_ptr(), float(reg), G_ptr, lam, Gsum_ptr, lam_cross,
-                                               ws.data_ptr(), ws_bytes, st), 'update_h')
+            if planes is None:
+                _lib.check(self._lib.tnmf_update_h(ctypes.byref(p), Vs.data_ptr(), R.data_ptr(), W.data_ptr(),
+                                                   Hs.data_ptr(), float(reg), G_ptr, lam, Gsum_ptr, lam_cross,
+                                                   ws.data_ptr(), ws_bytes, st), 'update_h')
+            else:
+                _lib.check(self._lib.tnmf_update_h_planes(ctypes.byref(p), Vs.data_ptr(), R.data_ptr(), W.data_ptr(),
+                                                          Hs.data_ptr(), float(reg), G_ptr, lam, Gsum_ptr, lam_cross,
+                                                          int(planes[0]), int(planes[1]), ws.data_ptr(), ws_bytes, st),
+                           'update_h_planes')
         self.launches += self._n_launches(p, _lib.OP_GRADIENT_H)
 
-    def gradient_W(self, V, W, H, s: slice, out: torch.Tensor, H_for_R: Optional[torch.Tensor] = None) -> torch.Tensor:
+    def gradient_W(self, V, W, H, s: slice, out: torch.Tensor, H_for_R: Optional[torch.Tensor] = None,
+                   planes: Optional[Tuple[int, int]] = None) -> torch.Tensor:
         """out[0] = neg, out[1] = pos of the W gradient on samples s (split-K + deterministic final reduction).
         `H_for_R`: reconstruct from these activations instead of H (halo sharding correlates with a band of H - the other
-        rows zeroed - against the reconstruction of all of it; tnmf_b200/halo.py)."""
+        rows zeroed - against the reconstruction of all of it; tnmf_b200/halo.py).
+        `planes=(t_lo, t_hi)`: correlate with those activation indices along the first shift axis only, as if H were zero
+        elsewhere, against the reconstruction of all of H (tnmf_gradient_w_planes; the same kernels as `update_H`'s)."""
         Hs = H[s]
         Vs = self._device_V(V)[s]
         n = Hs.shape[0]
@@ -591,9 +603,15 @@ class B200_Backend(Backend):  # pylint: disable=invalid-name
             p, Hs = self._h_problem(Hs)         # (reconstruct recorded the other tensor's problem)
         ws, ws_bytes = self._workspace(p)
         with self._timed('gradient_w'):
-            _lib.check(self._lib.tnmf_gradient_w(ctypes.byref(p), Vs.data_ptr(), R.data_ptr(), Hs.data_ptr(),
-                                                 out[0].data_ptr(), out[1].data_ptr(), ws.data_ptr(), ws_bytes,
-                                                 _stream_ptr(self.device)), 'gradient_w')
+            if planes is None:
+                _lib.check(self._lib.tnmf_gradient_w(ctypes.byref(p), Vs.data_ptr(), R.data_ptr(), Hs.data_ptr(),
+                                                     out[0].data_ptr(), out[1].data_ptr(), ws.data_ptr(), ws_bytes,
+                                                     _stream_ptr(self.device)), 'gradient_w')
+            else:
+                _lib.check(self._lib.tnmf_gradient_w_planes(ctypes.byref(p), Vs.data_ptr(), R.data_ptr(), Hs.data_ptr(),
+                                                            out[0].data_ptr(), out[1].data_ptr(), int(planes[0]),
+                                                            int(planes[1]), ws.data_ptr(), ws_bytes,
+                                                            _stream_ptr(self.device)), 'gradient_w_planes')
         self.launches += self._n_launches(p, _lib.OP_GRADIENT_W)
         return out
 

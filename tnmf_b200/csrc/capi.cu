@@ -535,6 +535,73 @@ int tnmf_gradient_w(const tnmf_problem *p, const void *V, const void *R, const v
                                       (double *)pos, st);
 }
 
+// The plane-window entry points: the kernels that serve them are the plane mode of the tensor-memory kernels (3-D float32
+// 'valid') and the generic kernels; every other family has no window and the call is unsupported.  The window is on the
+// first shift axis of the problem as the caller describes it (no rows view).
+static int window_family(const tnmf_problem *p, Geo &g, int op, int t_lo, int t_hi, int *family) {
+    int s = make_geo(p, g, false);
+    if (s) return s;
+    const int wax = 3 - p->ndim;
+    if (t_lo < 0 || t_hi < t_lo || t_hi > g.T[wax]) return TNMF_EINVAL;
+    *family = choose_family(p, g, op, &s);
+    if (s) return s;
+    if (*family == TNMF_PATH_GENERIC || (*family == TNMF_PATH_TC && plane_problem(g))) return TNMF_OK;
+    return TNMF_EUNSUPPORTED;
+}
+
+int tnmf_update_h_planes(const tnmf_problem *p, const void *V, const void *R, const void *W, void *H, double reg,
+                         const void *G, double lambda, const void *Gsum, double lambda_cross, int32_t t_lo, int32_t t_hi,
+                         void *workspace, size_t workspace_bytes, void *stream) {
+    (void)workspace; (void)workspace_bytes;
+    if (!H || !V || !R || !W) return TNMF_EINVAL;
+    if (lambda_cross != 0.0 && !Gsum) return TNMF_EINVAL;
+    if (lambda_cross == 0.0) Gsum = nullptr;
+    if (lambda == 0.0 && !Gsum) G = nullptr;
+    if ((lambda != 0.0 || Gsum) && !G) return TNMF_EINVAL;
+    Geo g;
+    int family;
+    int s = window_family(p, g, TNMF_OP_GRADIENT_H, t_lo, t_hi, &family);
+    if (s) return s;
+    if (g.N == 0 || t_lo == t_hi) return TNMF_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (family == TNMF_PATH_TC)
+        return tc_gradient_h_ts(g, (const float *)V, (const float *)R, (const float *)W, nullptr, nullptr, (float *)H, reg,
+                                (const float *)G, lambda, (const float *)Gsum, lambda_cross, st, t_lo, t_hi);
+    if (p->dtype == TNMF_F32)
+        return generic_gradient_h<float>(g, (const float *)V, (const float *)R, (const float *)W, nullptr, nullptr,
+                                         (float *)H, reg, (const float *)G, lambda, (const float *)Gsum, lambda_cross,
+                                         st, t_lo, t_hi);
+    return generic_gradient_h<double>(g, (const double *)V, (const double *)R, (const double *)W, nullptr, nullptr,
+                                      (double *)H, reg, (const double *)G, lambda, (const double *)Gsum, lambda_cross,
+                                      st, t_lo, t_hi);
+}
+
+int tnmf_gradient_w_planes(const tnmf_problem *p, const void *V, const void *R, const void *H, void *neg, void *pos,
+                           int32_t t_lo, int32_t t_hi, void *workspace, size_t workspace_bytes, void *stream) {
+    if (!V || !R || !H || !neg || !pos) return TNMF_EINVAL;
+    Geo g;
+    int family;
+    int s = window_family(p, g, TNMF_OP_GRADIENT_W, t_lo, t_hi, &family);
+    if (s) return s;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (g.N == 0) {
+        const size_t bytes = (size_t)g.M * g.C * (size_t)vol3(g.A) * (p->dtype == TNMF_F32 ? 4 : 8);
+        cudaError_t e = cudaMemsetAsync(neg, 0, bytes, st);
+        if (e == cudaSuccess) e = cudaMemsetAsync(pos, 0, bytes, st);
+        return status_from_cuda(e);
+    }
+    if (family == TNMF_PATH_TC) {
+        if (!workspace || workspace_bytes < tnmf_workspace_bytes(p)) return TNMF_EWORKSPACE;
+        return tc_gradient_w_ns(g, (const float *)V, (const float *)R, (const float *)H, (float *)neg, (float *)pos,
+                                workspace, workspace_bytes, st, t_lo, t_hi);
+    }
+    if (p->dtype == TNMF_F32)
+        return generic_gradient_w<float>(g, (const float *)V, (const float *)R, (const float *)H, (float *)neg,
+                                         (float *)pos, st, t_lo, t_hi);
+    return generic_gradient_w<double>(g, (const double *)V, (const double *)R, (const double *)H, (double *)neg,
+                                      (double *)pos, st, t_lo, t_hi);
+}
+
 int tnmf_update_w(const tnmf_problem *p, void *W, const void *neg, const void *pos, double eps, void *stream) {
     Geo g;
     int s = make_geo(p, g);

@@ -57,11 +57,13 @@ inline int status_from_cuda(cudaError_t e) { return e == cudaSuccess ? TNMF_OK :
 // ---- implemented in generic_kernels.cu -----------------------------------------------------------------
 template <typename T> int generic_reconstruct(const Geo &g, const T *W, const T *H, T *R, const T *V,
                                               double *energy_partials, int *n_partials, cudaStream_t st);
+// t_lo, t_hi: the window of activation indices [t_lo, t_hi) along the first shift axis that is updated / correlated
+// (t_hi < 0: all of them)
 template <typename T> int generic_gradient_h(const Geo &g, const T *V, const T *R, const T *W, T *neg, T *pos,
                                              T *H, double reg, const T *G, double lambda, const T *Gsum,
-                                             double lambda_cross, cudaStream_t st);
+                                             double lambda_cross, cudaStream_t st, int t_lo = 0, int t_hi = -1);
 template <typename T> int generic_gradient_w(const Geo &g, const T *V, const T *R, const T *H, T *neg, T *pos,
-                                             cudaStream_t st);
+                                             cudaStream_t st, int t_lo = 0, int t_hi = -1);
 int generic_energy_partial_capacity(const Geo &g);
 
 // ---- implemented in tiled_kernels.cu --------------------------------------------------------------------
@@ -113,8 +115,9 @@ int tc_gradient_w_ts(const Geo &g, const float *V, const float *R, const float *
 bool tc_gradw_ns_supported(const Geo &g, int dtype);
 size_t tc_gradw_ns_workspace_bytes(const Geo &g);
 int tc_gradw_ns_launches(const Geo &g);
+// t_lo, t_hi: 3-D only, correlate with the activation planes [t_lo, t_hi) only (t_hi < 0: all of them)
 int tc_gradient_w_ns(const Geo &g, const float *V, const float *R, const float *H, float *neg, float *pos, void *workspace,
-                     size_t workspace_bytes, cudaStream_t st);
+                     size_t workspace_bytes, cudaStream_t st, int t_lo = 0, int t_hi = -1);
 
 // ---- implemented in tc_recon.cu (tcgen05 3xTF32) ------------------------------------------------------------
 bool tc_recon_supported(const Geo &g, int dtype);
@@ -124,8 +127,10 @@ int tc_reconstruct(const Geo &g, const float *W, const float *H, float *R, const
 
 // ---- implemented in tc_hupd_ts.cu (tcgen05 3xTF32, expanded operand in tensor memory) ---------------------------
 bool tc_hupd_ts_supported(const Geo &g, int dtype);
+// t_lo, t_hi: 3-D only, update the activation planes [t_lo, t_hi) only (t_hi < 0: all of them)
 int tc_gradient_h_ts(const Geo &g, const float *V, const float *R, const float *W, float *neg, float *pos, float *H,
-                     double reg, const float *G, double lambda, const float *Gsum, double lambda_cross, cudaStream_t st);
+                     double reg, const float *G, double lambda, const float *Gsum, double lambda_cross, cudaStream_t st,
+                     int t_lo = 0, int t_hi = -1);
 
 // ---- implemented in tc_recon_ts.cu (tcgen05 3xTF32, activation row ring in tensor memory) ---------------------
 bool tc_recon_ts_supported(const Geo &g, int dtype);

@@ -74,21 +74,25 @@ generic_reconstruct_kernel(Geo g, const T *__restrict__ W, const T *__restrict__
 
 // neg/pos[n,m,t] = sum_c sum_a W[m,c,a] * Xext[n,c,t-off+a], X = V / R     (tnmf/backends/NumPy.py:93-120)
 // plus, when H is given, the fused multiplicative update (tnmf/TransformInvariantNMF.py:217-235,246-271).
+// Only the activation indices [t_lo, t_lo + E[wax]) along axis `wax` (the first shift axis) are visited; E is T elsewhere.
 template <typename T>
 __global__ void __launch_bounds__(kGenericThreads)
 generic_gradient_h_kernel(Geo g, const T *__restrict__ V, const T *__restrict__ R, const T *__restrict__ W,
                           T *__restrict__ neg_out, T *__restrict__ pos_out, T *__restrict__ H, T reg,
-                          const T *__restrict__ G, T lambda, const T *__restrict__ Gsum, T lambda_cross) {
+                          const T *__restrict__ G, T lambda, const T *__restrict__ Gsum, T lambda_cross,
+                          int wax, int t_lo, int t_n) {
     const long long dvol = vol3(g.D), avol = vol3(g.A), tvol = vol3(g.T);
-    const long long total = (long long)g.N * g.M * tvol;
-    for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total;
-         idx += (long long)gridDim.x * blockDim.x) {
-        long long r = idx;
-        const int tx = (int)(r % g.T[2]); r /= g.T[2];
-        const int ty = (int)(r % g.T[1]); r /= g.T[1];
-        const int tz = (int)(r % g.T[0]); r /= g.T[0];
+    const int E0 = wax == 0 ? t_n : g.T[0], E1 = wax == 1 ? t_n : g.T[1], E2 = wax == 2 ? t_n : g.T[2];
+    const long long total = (long long)g.N * g.M * E0 * E1 * E2;
+    for (long long w = (long long)blockIdx.x * blockDim.x + threadIdx.x; w < total;
+         w += (long long)gridDim.x * blockDim.x) {
+        long long r = w;
+        const int tx = (int)(r % E2) + (wax == 2 ? t_lo : 0); r /= E2;
+        const int ty = (int)(r % E1) + (wax == 1 ? t_lo : 0); r /= E1;
+        const int tz = (int)(r % E0) + (wax == 0 ? t_lo : 0); r /= E0;
         const int m = (int)(r % g.M);
         const int n = (int)(r / g.M);
+        const long long idx = (((long long)n * g.M + m) * g.T[0] + tz) * g.T[1] * g.T[2] + (long long)ty * g.T[2] + tx;
         T neg = 0, pos = 0;
         for (int c = 0; c < g.C; ++c) {
             const T *w = W + ((long long)m * g.C + c) * avol;
@@ -133,11 +137,12 @@ generic_gradient_h_kernel(Geo g, const T *__restrict__ V, const T *__restrict__ 
 }
 
 // neg/pos[m,c,a] = sum_n sum_d Hext[n,m,d+off-a] * X[n,c,d]               (tnmf/backends/NumPy.py:69-91)
-// One block per output element; the reduction runs in double.
+// One block per output element; the reduction runs in double.  Activation indices outside [t_lo, t_hi) along axis `wax`
+// (the first shift axis) do not contribute.
 template <typename T>
 __global__ void __launch_bounds__(kGenericThreads)
 generic_gradient_w_kernel(Geo g, const T *__restrict__ V, const T *__restrict__ R, const T *__restrict__ H,
-                          T *__restrict__ neg_out, T *__restrict__ pos_out) {
+                          T *__restrict__ neg_out, T *__restrict__ pos_out, int wax, int t_lo, int t_hi) {
     __shared__ double red[32];
     const long long dvol = vol3(g.D);
     long long r = blockIdx.x;
@@ -157,6 +162,8 @@ generic_gradient_w_kernel(Geo g, const T *__restrict__ V, const T *__restrict__ 
         int tz = z + g.off[0] - az, ty = y + g.off[1] - ay, tx = x + g.off[2] - ax;
         if (!fold_index(tz, g.T[0], g.wrap) || !fold_index(ty, g.T[1], g.wrap) || !fold_index(tx, g.T[2], g.wrap))
             continue;
+        const int tw = wax == 0 ? tz : wax == 1 ? ty : tx;
+        if (tw < t_lo || tw >= t_hi) continue;
         const double h = (double)H[n * g.hsn + m * g.hsm + ((long long)tz * g.T[1] + ty) * g.hsy + tx];
         const long long xi = ((long long)n * g.C + c) * dvol + ((long long)z * g.D[1] + y) * g.D[2] + x;
         neg += h * (double)V[xi];
@@ -190,19 +197,26 @@ int generic_reconstruct(const Geo &g, const T *W, const T *H, T *R, const T *V, 
 
 template <typename T>
 int generic_gradient_h(const Geo &g, const T *V, const T *R, const T *W, T *neg, T *pos, T *H, double reg,
-                       const T *G, double lambda, const T *Gsum, double lambda_cross, cudaStream_t st) {
-    const long long total = (long long)g.N * g.M * vol3(g.T);
+                       const T *G, double lambda, const T *Gsum, double lambda_cross, cudaStream_t st, int t_lo,
+                       int t_hi) {
+    const int wax = 3 - g.ndim;
+    if (t_hi < 0) { t_lo = 0; t_hi = g.T[wax]; }
+    if (t_hi <= t_lo) return TNMF_OK;
+    const long long total = (long long)g.N * g.M * (vol3(g.T) / g.T[wax]) * (t_hi - t_lo);
     generic_gradient_h_kernel<T><<<grid_for(total), kGenericThreads, 0, st>>>(
-        g, V, R, W, neg, pos, H, (T)reg, G, (T)lambda, Gsum, (T)lambda_cross);
+        g, V, R, W, neg, pos, H, (T)reg, G, (T)lambda, Gsum, (T)lambda_cross, wax, t_lo, t_hi - t_lo);
     TNMF_CHECK_LAUNCH();
     return TNMF_OK;
 }
 
 template <typename T>
-int generic_gradient_w(const Geo &g, const T *V, const T *R, const T *H, T *neg, T *pos, cudaStream_t st) {
+int generic_gradient_w(const Geo &g, const T *V, const T *R, const T *H, T *neg, T *pos, cudaStream_t st, int t_lo,
+                       int t_hi) {
     const long long outputs = (long long)g.M * g.C * vol3(g.A);
     if (outputs > 0x7fffffffLL) return TNMF_EUNSUPPORTED;
-    generic_gradient_w_kernel<T><<<(int)outputs, kGenericThreads, 0, st>>>(g, V, R, H, neg, pos);
+    const int wax = 3 - g.ndim;
+    if (t_hi < 0) { t_lo = 0; t_hi = g.T[wax]; }
+    generic_gradient_w_kernel<T><<<(int)outputs, kGenericThreads, 0, st>>>(g, V, R, H, neg, pos, wax, t_lo, t_hi);
     TNMF_CHECK_LAUNCH();
     return TNMF_OK;
 }
@@ -211,8 +225,8 @@ int generic_gradient_w(const Geo &g, const T *V, const T *R, const T *H, T *neg,
     template int generic_reconstruct<T>(const Geo &, const T *, const T *, T *, const T *, double *, int *,      \
                                         cudaStream_t);                                                          \
     template int generic_gradient_h<T>(const Geo &, const T *, const T *, const T *, T *, T *, T *, double,      \
-                                       const T *, double, const T *, double, cudaStream_t);                     \
-    template int generic_gradient_w<T>(const Geo &, const T *, const T *, const T *, T *, T *, cudaStream_t);
+                                       const T *, double, const T *, double, cudaStream_t, int, int);           \
+    template int generic_gradient_w<T>(const Geo &, const T *, const T *, const T *, T *, T *, cudaStream_t, int, int);
 INSTANTIATE(float)
 INSTANTIATE(double)
 

@@ -37,8 +37,13 @@ using tma::smem_u32;
 //   H plane t of sample n, atom m:         n * hsn + m * hsm + t * hsz
 // The reconstruction and the W gradient launch once per a_z (NZ = D_z, H shifted by offz - az planes); the H update
 // launches once, its a_z planes being extra channels (c, a_z) of the contraction (NZ = T_z, Geo2::C = C * A_z).
+// A plane window (tnmf_update_h_planes / tnmf_gradient_w_planes) runs over the virtual samples (n, z0 + z'), z' < NZ: the
+// H update over the activation planes [z0, z0 + NZ) = [t_lo, t_hi), each W-gradient launch over the sample planes whose
+// activation plane lies in the window.  Every address and boundary test uses the absolute plane z0 + z'.
 struct Geo3 : tiled::Geo2 {
     int NZ;                 // planes per sample in the virtual sample index
+    int z0;                 // absolute plane of z' = 0 (0 without a window)
+    int TZ;                 // activation planes of the whole problem (the pitch of the dense G / Gsum inputs)
     int DZ, AZ, offz;       // sample planes, atom planes, A_z - 1
     int az;                 // atom plane of this launch (reconstruction, W gradient)
     int acc;                // reconstruction: add to R instead of writing it (every launch after the first)
@@ -59,6 +64,8 @@ inline Geo3 make_geo3(const Geo &g, bool h_update, int az = 0) {
     static_cast<tiled::Geo2 &>(q) = tiled::make_geo2(g);
     q.NZ = h_update ? g.T[0] : g.D[0];
     q.N = g.N * q.NZ;
+    q.z0 = 0;
+    q.TZ = g.T[0];
     if (h_update) q.C = g.C * g.A[0];
     q.DZ = g.D[0]; q.AZ = g.A[0]; q.offz = g.off[0];
     q.az = az; q.acc = 0;
@@ -66,6 +73,12 @@ inline Geo3 make_geo3(const Geo &g, bool h_update, int az = 0) {
     q.xsn = q.xsc * g.C;
     q.hsz = (long long)g.T[1] * g.hsy;
     return q;
+}
+// the same geometry restricted to the planes [z0, z0 + nz) of the virtual sample index
+inline void window_geo3(Geo3 &q, int n_samples, int z0, int nz) {
+    q.z0 = z0;
+    q.NZ = nz;
+    q.N = n_samples * nz;
 }
 
 // Wait with back-off for roles that are far from the critical path: every poll of a spinning warp is a shared-memory

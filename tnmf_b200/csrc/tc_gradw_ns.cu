@@ -65,7 +65,9 @@ struct Args {
     int m0;
 };
 
-bool make_plan(const Geo2 &g, Plan &p) {
+// max_grid > 0: at most that many CTAs (longer ranges per CTA), so that the partial slices fit a workspace planned
+// for a larger problem
+bool make_plan(const Geo2 &g, Plan &p, int max_grid = 0) {
     p = Plan();
     if (g.AY < 1 || g.AY > 19) return false;
     p.KPL = g.C * g.AX;
@@ -107,6 +109,7 @@ bool make_plan(const Geo2 &g, Plan &p) {
     p.quota = (p.total + sms - 1) / sms;
     const long long min_quota = g.TY < 8 ? g.TY : 8;
     if (p.quota < min_quota) p.quota = min_quota;
+    if (max_grid > 0 && (p.total + p.quota - 1) / p.quota > max_grid) p.quota = (p.total + max_grid - 1) / max_grid;
     p.grid = (int)((p.total + p.quota - 1) / p.quota);
     p.units = (long long)p.grid * ((p.quota + g.TY - 2) / g.TY + 1);
     return true;
@@ -211,7 +214,7 @@ __device__ __forceinline__ void gradw_ns_body(const G &g, const Plan &p, const A
                     const int n = (int)(J / p.TXP);
                     const int x = (int)(J - (long long)n * p.TXP) - g.offx;
                     if (n < g.N && (unsigned)x < (unsigned)g.DX) {
-                        if constexpr (P3) roff[e] = (n / g.NZ) * g.xsn + c * g.xsc + (long long)(n % g.NZ) * plane + x;
+                        if constexpr (P3) roff[e] = (n / g.NZ) * g.xsn + c * g.xsc + (long long)(g.z0 + n % g.NZ) * plane + x;
                         else roff[e] = ((long long)n * C + c) * plane + x;
                     }
                 }
@@ -223,7 +226,7 @@ __device__ __forceinline__ void gradw_ns_body(const G &g, const Plan &p, const A
                 const int n = (int)(J / p.TXP);
                 const int xv = (int)(J - (long long)n * p.TXP);
                 long long hbase;
-                if constexpr (P3) hbase = (long long)(n / g.NZ) * g.hsn + (long long)(n % g.NZ) * g.hsz;
+                if constexpr (P3) hbase = (long long)(n / g.NZ) * g.hsn + (long long)(g.z0 + n % g.NZ) * g.hsz;
                 else hbase = (long long)n * g.hsn;
                 hoff[e] = (n < g.N && xv < g.TX && a.m0 + h_ml < g.M) ? hbase + (long long)(a.m0 + h_ml) * g.hsm + xv : -1;
             }
@@ -503,7 +506,7 @@ size_t tc_gradw_ns_workspace_bytes(const Geo &g) {
 }
 
 int tc_gradient_w_ns(const Geo &g, const float *V, const float *R, const float *H, float *neg, float *pos, void *workspace,
-                     size_t workspace_bytes, cudaStream_t st) {
+                     size_t workspace_bytes, cudaStream_t st, int t_lo, int t_hi) {
     const bool planes = plane_problem(g);
     tc::Geo3 q3 = tc::make_geo3(g, false);
     const tiled::Geo2 q = planes ? q3 : tiled::make_geo2(g);
@@ -518,14 +521,31 @@ int tc_gradient_w_ns(const Geo &g, const float *V, const float *R, const float *
     cudaError_t e = cudaFuncSetAttribute(planes ? (const void *)kern3 : (const void *)kern,
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, tc::gwn::kMaxSmem);
     if (e != cudaSuccess) return status_from_cuda(e);
+    // A plane window [t_lo, t_hi): the pass of a_z covers the sample planes z whose activation plane z + offz - a_z lies
+    // in it.  Its own plan has at most p.grid CTAs, and the CTAs (and a_z slices) it leaves out must read as zeros in the
+    // fixed-order reduction over the p.grid * 4 slices: the partials are cleared first.  (The full window runs the
+    // unwindowed launches.)
+    const bool window = t_hi >= 0 && !(t_lo <= 0 && t_hi >= g.T[0]);
+    if (window && !planes) return TNMF_EUNSUPPORTED;
+    if (window) {
+        cudaError_t e = cudaMemsetAsync(workspace, 0, tc_gradw_ns_workspace_bytes(g), st);
+        if (e != cudaSuccess) return status_from_cuda(e);
+    }
     // 3-D: one pass per atom plane a_z over the virtual samples (n, z), against H shifted by offz - a_z planes; each pass
     // fills its own a_z slice of every partial, and one fixed-order reduction finishes all of them
     for (int az = 0; az < (planes ? g.A[0] : 1); ++az) {
         q3.az = az;
         a.H = planes ? H + (long long)(q3.offz - az) * q3.hsz : H;
+        tc::gwn::Plan pz = p;
+        if (window) {
+            const int z0 = max(0, t_lo - q3.offz + az), z1 = min(g.D[0], t_hi - q3.offz + az);
+            if (z1 <= z0) continue;
+            tc::window_geo3(q3, g.N, z0, z1 - z0);
+            if (!tc::gwn::make_plan(q3, pz, p.grid)) return TNMF_EUNSUPPORTED;
+        }
         for (int m0 = 0; m0 < g.M; m0 += tc::gwn::kNB) {
             a.m0 = m0;
-            if (planes) kern3<<<(unsigned)p.grid, tc::gwn::kThreads, p.smem, st>>>(q3, p, a);
+            if (planes) kern3<<<(unsigned)pz.grid, tc::gwn::kThreads, pz.smem, st>>>(q3, pz, a);
             else kern<<<(unsigned)p.grid, tc::gwn::kThreads, p.smem, st>>>(q, p, a);
             TNMF_CHECK_LAUNCH();
         }

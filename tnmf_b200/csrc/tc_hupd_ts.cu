@@ -208,7 +208,7 @@ __device__ __forceinline__ void hupd_ts_body(const G &g, const Plan &p, const Ar
                     const int x = (int)(J - (long long)n * p.TXP) - g.offx;
                     if (n < g.N && (unsigned)x < (unsigned)g.DX) {
                         if constexpr (P3) {
-                            const int ns = n / g.NZ, cr = c / g.AZ, z = n - ns * g.NZ - g.offz + (c - cr * g.AZ);
+                            const int ns = n / g.NZ, cr = c / g.AZ, z = g.z0 + n - ns * g.NZ - g.offz + (c - cr * g.AZ);
                             if ((unsigned)z < (unsigned)g.DZ) roff[e] = ns * g.xsn + cr * g.xsc + (long long)z * plane + x;
                         } else {
                             roff[e] = ((long long)n * C + c) * plane + x;
@@ -304,7 +304,7 @@ __device__ __forceinline__ void hupd_ts_body(const G &g, const Plan &p, const Ar
             // the activations of a row do not depend on the accumulators: they are fetched one row ahead
             float hnext[kHA];
             long long hbase;
-            if constexpr (P3) hbase = (long long)(n / g.NZ) * g.hsn + (long long)(n % g.NZ) * g.hsz;
+            if constexpr (P3) hbase = (long long)(n / g.NZ) * g.hsn + (long long)(g.z0 + n % g.NZ) * g.hsz;
             else hbase = (long long)n * g.hsn;
             float *hrow = (a.H && active) ? a.H + hbase + (long long)ma * g.hsm + tx : nullptr;
             auto load_h = [&](int ty) {
@@ -365,8 +365,8 @@ __device__ __forceinline__ void hupd_ts_body(const G &g, const Plan &p, const Ar
                 for (int ml = 0; ml < kHA; ++ml) {
                     const int m = ma + ml;
                     if (m >= g.M) continue;
-                    long long cidx;                 // dense [n][m][(t_z,) t_y][t_x]; Gsum has one atom: n * tvol suits both
-                    if constexpr (P3) cidx = (((long long)(n / g.NZ) * g.M + m) * g.NZ + n % g.NZ) * tvol + tin;
+                    long long cidx;                 // dense [n][m][(t_z,) t_y][t_x] of the whole problem
+                    if constexpr (P3) cidx = (((long long)(n / g.NZ) * g.M + m) * g.TZ + g.z0 + n % g.NZ) * tvol + tin;
                     else cidx = ((long long)n * g.M + m) * tvol + tin;
                     if (a.H) {
                         const float h = hv[ml];
@@ -375,7 +375,10 @@ __device__ __forceinline__ void hupd_ts_body(const G &g, const Plan &p, const Ar
                             const float gv = a.G[cidx];
                             if (a.lambda != 0.f) { float tmp = gv - h; tmp *= a.lambda; ps += tmp; }
                             if (a.Gsum) {
-                                const float gs = a.Gsum[(long long)n * tvol + tin];
+                                long long sidx;         // Gsum: one atom
+                                if constexpr (P3) sidx = ((long long)(n / g.NZ) * g.TZ + g.z0 + n % g.NZ) * tvol + tin;
+                                else sidx = (long long)n * tvol + tin;
+                                const float gs = a.Gsum[sidx];
                                 float tmp = -gv + gs; tmp *= a.lambda_cross; ps += tmp;
                             }
                         }
@@ -561,11 +564,19 @@ static int gradient_h_ts(const G &q, int M, const float *V, const float *R, cons
 }
 
 int tc_gradient_h_ts(const Geo &g, const float *V, const float *R, const float *W, float *neg, float *pos, float *H,
-                     double reg, const float *G, double lambda, const float *Gsum, double lambda_cross, cudaStream_t st) {
+                     double reg, const float *G, double lambda, const float *Gsum, double lambda_cross, cudaStream_t st,
+                     int t_lo, int t_hi) {
     // 3-D: ONE launch per block of atoms - the a_z planes are channels of the contraction, so the fused epilogue sees
-    // complete sums
-    if (plane_problem(g))
-        return gradient_h_ts(tc::make_geo3(g, true), g.M, V, R, W, neg, pos, H, reg, G, lambda, Gsum, lambda_cross, st);
+    // complete sums.  A plane window [t_lo, t_hi) makes the virtual samples (n, t_lo + t'), t' < t_hi - t_lo.
+    if (plane_problem(g)) {
+        tc::Geo3 q = tc::make_geo3(g, true);
+        if (t_hi >= 0) {
+            if (t_hi <= t_lo) return TNMF_OK;
+            tc::window_geo3(q, g.N, t_lo, t_hi - t_lo);
+        }
+        return gradient_h_ts(q, g.M, V, R, W, neg, pos, H, reg, G, lambda, Gsum, lambda_cross, st);
+    }
+    if (t_hi >= 0) return TNMF_EUNSUPPORTED;
     return gradient_h_ts(tiled::make_geo2(g), g.M, V, R, W, neg, pos, H, reg, G, lambda, Gsum, lambda_cross, st);
 }
 
