@@ -294,18 +294,21 @@ class B200_Backend(Backend):  # pylint: disable=invalid-name
     def buffer_pointers(self) -> tuple:
         return tuple(t.data_ptr() for t in self.buffer_tensors())
 
+    def _planned_problem(self, n: Optional[int]) -> _lib.Problem:
+        """The last problem run (n None), or a batch of `n` samples laid out the way `initialize` would lay it out."""
+        if n is None:
+            return self._last_h_problem
+        shape = (int(n), self.n_atoms, *self._transform_shape)
+        pad = self._h_padding(shape)
+        hsm = int(np.prod(shape[2:-1], dtype=np.int64)) * (shape[-1] + pad)
+        return self._problem(int(n), self.n_atoms, self.n_atoms * hsm, hsm,
+                             (shape[-1] + pad) if pad and len(self.atom_shape) >= 2 else 0)
+
     def kernel_families(self, n: Optional[int] = None) -> dict:
         """Which kernel family (generic / tiled / tma / tc) serves each hot-path operation: of the last problem run, or
         of a batch of `n` samples laid out the way `initialize` would (nothing is allocated)."""
         names = {v: k for k, v in _lib.PATHS.items()}
-        if n is None:
-            p = self._last_h_problem
-        else:
-            shape = (int(n), self.n_atoms, *self._transform_shape)
-            pad = self._h_padding(shape)
-            hsm = int(np.prod(shape[2:-1], dtype=np.int64)) * (shape[-1] + pad)
-            p = self._problem(int(n), self.n_atoms, self.n_atoms * hsm, hsm,
-                              (shape[-1] + pad) if pad and len(self.atom_shape) >= 2 else 0)
+        p = self._planned_problem(n)
         return {op: names.get(int(self._lib.tnmf_kernel_family(ctypes.byref(p), code)), 'none')
                 for op, code in (('reconstruct', _lib.OP_RECONSTRUCT), ('update_h', _lib.OP_GRADIENT_H),
                                  ('gradient_w', _lib.OP_GRADIENT_W))}
@@ -313,14 +316,7 @@ class B200_Backend(Backend):  # pylint: disable=invalid-name
     def kernel_names(self, n: Optional[int] = None) -> dict:
         """The hot kernel (__global__ function name, as an ncu launch list shows it) behind each operation; arguments as
         for `kernel_families`."""
-        if n is None:
-            p = self._last_h_problem
-        else:
-            shape = (int(n), self.n_atoms, *self._transform_shape)
-            pad = self._h_padding(shape)
-            hsm = int(np.prod(shape[2:-1], dtype=np.int64)) * (shape[-1] + pad)
-            p = self._problem(int(n), self.n_atoms, self.n_atoms * hsm, hsm,
-                              (shape[-1] + pad) if pad and len(self.atom_shape) >= 2 else 0)
+        p = self._planned_problem(n)
         return {op: self._lib.tnmf_kernel_name(ctypes.byref(p), code).decode()
                 for op, code in (('reconstruct', _lib.OP_RECONSTRUCT), ('update_h', _lib.OP_GRADIENT_H),
                                  ('gradient_w', _lib.OP_GRADIENT_W))}

@@ -1,4 +1,4 @@
-// extern "C" surface of libtnmf_b200.so: argument validation, geometry set-up and kernel-family dispatch.
+// extern "C" surface of libtnmf_b200.so: argument validation, geometry set-up, kernel choice and dispatch.
 // See include/tnmf_b200.h for the contract of every entry point and the reference interface it replaces.
 #include <cstdio>
 #include <cstdlib>
@@ -92,40 +92,19 @@ bool tc_gradw_worthwhile(const Geo &g) {
            g.A[1] >= 3 && g.A[1] <= 15;
 }
 
-// Tensor-core kernels whose expanded operand lives in tensor memory (tc_*_ts.cu) take over wherever they plan
-bool tmem_operand_hupd(const Geo &g, int dtype) {
-    return !(g.flags & TNMF_FLAG_NO_TMEM_OPERAND) && tc_hupd_ts_supported(g, dtype);
-}
-bool tmem_operand_gradw(const Geo &g, int dtype) {
-    return !(g.flags & TNMF_FLAG_NO_TMEM_OPERAND) && tc_gradw_ts_supported(g, dtype);
-}
-
 // The W gradient for narrow atoms (tc_gradw_ns.cu: C * A_x <= 16; hi / lo halves, two source rows and both tensors stacked
 // in the 128 MMA lanes, two MMAs per product): 'auto' takes it when at least half of the lanes carry taps.
-bool tmem_operand_gradw_ns(const Geo &g, int dtype) {
-    return !(g.flags & TNMF_FLAG_NO_TMEM_OPERAND) && tc_gradw_ns_supported(g, dtype);
-}
 bool tc_gradw_ns_worthwhile(const Geo &g) {
     if (g.flags & TNMF_FLAG_NO_TC_GRADW) return false;
     const int mp = (g.M + 7) / 8 * 8;
     return 8 * g.C * g.A[2] >= 64 && (double)g.M / mp >= 0.5 && (long long)g.N * g.T[2] >= 64 && g.A[1] >= 3;
 }
-// which of the three tensor-core W gradients serves a problem whose family is TNMF_PATH_TC
-enum { GRADW_NS = 0, GRADW_TS = 1, GRADW_SS = 2 };
-int tc_gradw_variant(const tnmf_problem *p, const Geo &g) {
-    if (plane_problem(g)) return GRADW_NS;
-    const bool forced = p->path == TNMF_PATH_TC;
-    if (tmem_operand_gradw_ns(g, p->dtype) && (forced || tc_gradw_ns_worthwhile(g))) return GRADW_NS;
-    if (tmem_operand_gradw(g, p->dtype)) return GRADW_TS;
-    return GRADW_SS;
-}
 
-// The reconstruction with the activation row ring in tensor memory: N = roundup(C * A_x, 16), K = atoms padded to 8, and
-// 128 - (A_x - 1) of the 128 MMA lanes produce outputs; 'auto' takes it when at least half of every MMA is useful work.
-bool tmem_operand_recon(const Geo &g, int dtype) {
-    return !(g.flags & TNMF_FLAG_NO_TMEM_OPERAND) && tc_recon_ts_supported(g, dtype);
-}
-bool tc_recon_ts_worthwhile(const Geo &g) {
+// The reconstructions with a tensor-memory ring - of activation rows (tc_recon_ts.cu: N = roundup(C * A_x, 16)) or, for
+// what that kernel cannot hold (one channel, many atoms: cfg3), of output-row accumulators (tc_recon_os.cu: one MMA of
+// N = A_y * roundup(C * A_x, 16) per source row and K step).  K = atoms padded to 8, and 128 - (A_x - 1) of the 128 MMA
+// lanes produce outputs; 'auto' takes them when at least half of every MMA is useful work.
+bool tc_recon_tmem_worthwhile(const Geo &g) {
     if (g.flags & TNMF_FLAG_NO_TC_RECON) return false;
     const int nu = g.C * g.A[2], np = (nu + 15) / 16 * 16, km = (g.M + 7) / 8 * 8;
     const double useful = ((double)nu / np) * ((double)g.M / km) * (double)(128 - (g.A[2] - 1)) / 128.0;
@@ -133,87 +112,78 @@ bool tc_recon_ts_worthwhile(const Geo &g) {
     return useful >= 0.5 && (long long)g.N * g.D[2] >= 128 && g.A[1] >= 3;
 }
 
-// The reconstruction for narrow atoms (tc_recon_os.cu: output rows as a ring of accumulators in tensor memory, one MMA of
-// N = A_y * roundup(C * A_x, 16) per source row and K step) serves what the activation-ring kernel cannot hold - one
-// channel, many atoms (cfg3).  'auto' takes it when at least half of every MMA is useful work.
-bool tmem_operand_recon_os(const Geo &g, int dtype) {
-    return !(g.flags & TNMF_FLAG_NO_TMEM_OPERAND) && tc_recon_os_supported(g, dtype);
-}
-bool tc_recon_os_worthwhile(const Geo &g) {
-    if (g.flags & TNMF_FLAG_NO_TC_RECON) return false;
-    const int nu = g.C * g.A[2], np = (nu + 15) / 16 * 16, km = (g.M + 7) / 8 * 8;
-    const double useful = ((double)nu / np) * ((double)g.M / km) * (double)(128 - (g.A[2] - 1)) / 128.0;
-    return useful >= 0.5 && (long long)g.N * g.D[2] >= 128 && g.A[1] >= 3;
-}
-// which of the three tensor-core reconstructions serves a problem whose family is TNMF_PATH_TC
-enum { RECON_TS = 0, RECON_OS = 1, RECON_SS = 2 };
-int tc_recon_variant(const tnmf_problem *p, const Geo &g) {
-    if (plane_problem(g)) return RECON_OS;
-    const bool forced = p->path == TNMF_PATH_TC;
-    if (tmem_operand_recon(g, p->dtype) && (forced || tc_recon_ts_worthwhile(g))) return RECON_TS;
-    if (tmem_operand_recon_os(g, p->dtype) && (forced || tc_recon_os_worthwhile(g))) return RECON_OS;
-    return RECON_SS;
-}
+// Every hot kernel an operation can run on.  The FP32 and generic families have one kernel per operation and share the
+// values of their TNMF_PATH_*; every other value is a tensor-core kernel (family TNMF_PATH_TC).
+enum Kernel {
+    K_NONE = -1,
+    K_GENERIC = TNMF_PATH_GENERIC, K_TILED = TNMF_PATH_TILED, K_TMA = TNMF_PATH_TMA,
+    K_RECON_TS = TNMF_PATH_TC, K_RECON_OS, K_RECON_TC, K_HUPD_TS, K_HUPD_TC, K_GRADW_TS, K_GRADW_NS, K_GRADW_TC,
+    K_RECON_OS3, K_HUPD_TS3, K_GRADW_NS3,                      // the 3-D plane mode of recon_os, hupd_ts and gradw_ns
+};
 
-// 3-D problems (three shift axes in use) run on the plane mode of three tensor-memory kernels (DESIGN.md §3.10):
-// hupd_ts, recon_os (C <= 2) and gradw_ns (C * A_x <= 16), float32 'valid' only.  Their alternative is the generic
-// kernel, not the FP32 tiled / TMA ones (2-D only), so 'auto' takes them wherever they plan and at least half of every
-// 16-atom block is real atoms (a few atoms in a large padded MMA lose to nothing).  The TNMF_FLAG_NO_TC_* flags keep
-// 'auto' on the generic kernels, TNMF_FLAG_NO_TMEM_OPERAND keeps every path there.
-bool planes_tc(const tnmf_problem *p, const Geo &g, int op) {
-    if (g.flags & TNMF_FLAG_NO_TMEM_OPERAND) return false;
-    if (p->path == TNMF_PATH_AUTO) {
-        const int off = op == TNMF_OP_RECONSTRUCT ? TNMF_FLAG_NO_TC_RECON
-                      : op == TNMF_OP_GRADIENT_H  ? TNMF_FLAG_NO_TC_HUPD : TNMF_FLAG_NO_TC_GRADW;
-        if ((g.flags & off) || (double)g.M / ((g.M + 15) / 16 * 16) < 0.5) return false;
-    } else if (p->path != TNMF_PATH_TC) {
-        return false;
-    }
-    if (op == TNMF_OP_RECONSTRUCT) return tc_recon_os_supported(g, p->dtype);
-    if (op == TNMF_OP_GRADIENT_H) return tc_hupd_ts_supported(g, p->dtype);
-    return tc_gradw_ns_supported(g, p->dtype);
-}
+int kernel_family(int k) { return k < TNMF_PATH_TC ? k : TNMF_PATH_TC; }
 
-// Kernel family serving operation `op`: TMA where eligible, else the cp.async tiled kernels, else the generic ones;
-// a forced family that cannot serve the problem is an error.
-int choose_family(const tnmf_problem *p, const Geo &g, int op, int *err) {
+// The kernel that serves operation `op`, or K_NONE with *err set when a forced family cannot serve the problem.  'auto'
+// takes a tensor-core kernel where it plans and is worthwhile, the tensor-memory operand kernels before the round-1 ones;
+// else the TMA kernels where eligible, else the cp.async tiled ones, else the generic ones.  Forced 'tc' takes a
+// tensor-core kernel wherever one plans and otherwise goes on like 'auto'.
+int plan_kernel(const tnmf_problem *p, const Geo &g, int op, int *err) {
     *err = TNMF_OK;
-    if (p->path == TNMF_PATH_GENERIC) return TNMF_PATH_GENERIC;
-    if (plane_problem(g)) {                                     // (the tiled and TMA kernels are 2-D only)
-        if (planes_tc(p, g, op)) return TNMF_PATH_TC;
-        if (p->path == TNMF_PATH_TMA || p->path == TNMF_PATH_TILED) { *err = TNMF_EUNSUPPORTED; return -1; }
-        return TNMF_PATH_GENERIC;                                   // forced 'tc': tensor cores where a kernel plans
+    if (p->path == TNMF_PATH_GENERIC) return K_GENERIC;
+    const int dt = p->dtype;
+    const bool forced = p->path == TNMF_PATH_TC, autop = p->path == TNMF_PATH_AUTO;
+    const bool tmem = !(g.flags & TNMF_FLAG_NO_TMEM_OPERAND);
+    if (plane_problem(g)) {
+        // 3-D problems run on the plane mode of three tensor-memory kernels (DESIGN.md §3.10), float32 'valid' only.
+        // Their alternative is the generic kernel, not the FP32 tiled / TMA ones (2-D only), so 'auto' takes them
+        // wherever they plan and at least half of every 16-atom block is real atoms (a few atoms in a large padded MMA
+        // lose to nothing).  The TNMF_FLAG_NO_TC_* flags keep 'auto' on the generic kernels, TNMF_FLAG_NO_TMEM_OPERAND
+        // keeps every path there.
+        static const int no_tc[3] = {TNMF_FLAG_NO_TC_RECON, TNMF_FLAG_NO_TC_HUPD, TNMF_FLAG_NO_TC_GRADW};
+        if (tmem && (forced || (autop && !(g.flags & no_tc[op]) && (double)g.M / ((g.M + 15) / 16 * 16) >= 0.5))) {
+            if (op == TNMF_OP_RECONSTRUCT && tc_recon_os_supported(g, dt)) return K_RECON_OS3;
+            if (op == TNMF_OP_GRADIENT_H && tc_hupd_ts_supported(g, dt)) return K_HUPD_TS3;
+            if (op == TNMF_OP_GRADIENT_W && tc_gradw_ns_supported(g, dt)) return K_GRADW_NS3;
+        }
+        if (p->path == TNMF_PATH_TMA || p->path == TNMF_PATH_TILED) { *err = TNMF_EUNSUPPORTED; return K_NONE; }
+        return K_GENERIC;                                           // forced 'tc': tensor cores where a kernel plans
     }
-    if (op == TNMF_OP_GRADIENT_H && (p->path == TNMF_PATH_TC || (p->path == TNMF_PATH_AUTO && tc_worthwhile(g))) &&
-        (tc_hupd_supported(g, p->dtype) || tmem_operand_hupd(g, p->dtype)))
-        return TNMF_PATH_TC;
-    if (op == TNMF_OP_RECONSTRUCT && tmem_operand_recon(g, p->dtype) &&
-        (p->path == TNMF_PATH_TC || (p->path == TNMF_PATH_AUTO && tc_recon_ts_worthwhile(g))))
-        return TNMF_PATH_TC;
-    if (op == TNMF_OP_RECONSTRUCT && tmem_operand_recon_os(g, p->dtype) &&
-        (p->path == TNMF_PATH_TC || (p->path == TNMF_PATH_AUTO && tc_recon_os_worthwhile(g))))
-        return TNMF_PATH_TC;
-    if (op == TNMF_OP_RECONSTRUCT && (p->path == TNMF_PATH_TC || (p->path == TNMF_PATH_AUTO && tc_recon_worthwhile(g))) &&
-        tc_recon_supported(g, p->dtype))
-        return TNMF_PATH_TC;
-    if (op == TNMF_OP_GRADIENT_W && tmem_operand_gradw_ns(g, p->dtype) &&
-        (p->path == TNMF_PATH_TC || (p->path == TNMF_PATH_AUTO && tc_gradw_ns_worthwhile(g))))
-        return TNMF_PATH_TC;
-    if (op == TNMF_OP_GRADIENT_W && (p->path == TNMF_PATH_TC || (p->path == TNMF_PATH_AUTO && tc_gradw_worthwhile(g))) &&
-        (tc_gradw_supported(g, p->dtype) || tmem_operand_gradw(g, p->dtype)))
-        return TNMF_PATH_TC;
     bool tma_ok = false;
-    if (p->path == TNMF_PATH_AUTO || p->path == TNMF_PATH_TMA || p->path == TNMF_PATH_TC) {
-        if (op == TNMF_OP_RECONSTRUCT) tma_ok = tma_recon_supported(g, p->dtype);
-        else if (op == TNMF_OP_GRADIENT_H) tma_ok = tma_hupd_supported(g, p->dtype);
-        else tma_ok = tma_gradw_supported(g, p->dtype);
+    if (op == TNMF_OP_RECONSTRUCT) {
+        const bool tmem_want = forced || (autop && tc_recon_tmem_worthwhile(g));
+        if (tmem && tmem_want && tc_recon_ts_supported(g, dt)) return K_RECON_TS;
+        if (tmem && tmem_want && tc_recon_os_supported(g, dt)) return K_RECON_OS;
+        if ((forced || (autop && tc_recon_worthwhile(g))) && tc_recon_supported(g, dt)) return K_RECON_TC;
+        tma_ok = tma_recon_supported(g, dt);
+    } else if (op == TNMF_OP_GRADIENT_H) {
+        if (forced || (autop && tc_worthwhile(g))) {
+            if (tmem && tc_hupd_ts_supported(g, dt)) return K_HUPD_TS;
+            if (tc_hupd_supported(g, dt)) return K_HUPD_TC;
+        }
+        tma_ok = tma_hupd_supported(g, dt);
+    } else {
+        if (tmem && (forced || (autop && tc_gradw_ns_worthwhile(g))) && tc_gradw_ns_supported(g, dt)) return K_GRADW_NS;
+        if (forced || (autop && tc_gradw_worthwhile(g))) {
+            if (tmem && tc_gradw_ts_supported(g, dt)) return K_GRADW_TS;
+            if (tc_gradw_supported(g, dt)) return K_GRADW_TC;
+        }
+        tma_ok = tma_gradw_supported(g, dt);
     }
-    if (tma_ok) return TNMF_PATH_TMA;
-    if (p->path == TNMF_PATH_TMA) { *err = TNMF_EUNSUPPORTED; return -1; }
-    const bool tiled_ok = tiled_supported(g, p->dtype);
-    if (tiled_ok) return TNMF_PATH_TILED;
-    if (p->path == TNMF_PATH_TILED) { *err = TNMF_EUNSUPPORTED; return -1; }
-    return TNMF_PATH_GENERIC;
+    if (tma_ok && (autop || forced || p->path == TNMF_PATH_TMA)) return K_TMA;
+    if (p->path == TNMF_PATH_TMA) { *err = TNMF_EUNSUPPORTED; return K_NONE; }
+    if (tiled_supported(g, dt)) return K_TILED;
+    if (p->path == TNMF_PATH_TILED) { *err = TNMF_EUNSUPPORTED; return K_NONE; }
+    return K_GENERIC;
+}
+
+// The TMA kernels need 16-byte aligned operands (`aligned`: those the caller's kernel reads) and a workspace for the
+// pre-arranged atoms: without them a forced 'tma' is an error, and the other paths fall back to the tiled kernels, else
+// the generic ones.
+int tma_fallback(const tnmf_problem *p, const Geo &g, int &k, bool aligned, bool workspace) {
+    if (k != K_TMA || (aligned && workspace)) return TNMF_OK;
+    if (p->path == TNMF_PATH_TMA) return workspace ? TNMF_EUNSUPPORTED : TNMF_EWORKSPACE;
+    k = tiled_supported(g, p->dtype) ? K_TILED : K_GENERIC;
+    return TNMF_OK;
 }
 
 size_t align256(size_t b) { return (b + 255) & ~(size_t)255; }
@@ -296,8 +266,8 @@ int tnmf_uses_tiled_path(const tnmf_problem *p) {
     Geo g;
     if (make_geo(p, g)) return 0;
     int err;
-    const int f = choose_family(p, g, TNMF_OP_GRADIENT_H, &err);
-    return (f == TNMF_PATH_TILED || f == TNMF_PATH_TMA || f == TNMF_PATH_TC) ? 1 : 0;
+    const int k = plan_kernel(p, g, TNMF_OP_GRADIENT_H, &err);
+    return k != K_NONE && k != K_GENERIC;
 }
 
 int tnmf_kernel_family(const tnmf_problem *p, int op) {
@@ -305,31 +275,33 @@ int tnmf_kernel_family(const tnmf_problem *p, int op) {
     if (make_geo(p, g)) return -1;
     if (op < TNMF_OP_RECONSTRUCT || op > TNMF_OP_GRADIENT_W) return -1;
     int err;
-    return choose_family(p, g, op, &err);
+    return kernel_family(plan_kernel(p, g, op, &err));
 }
 
 const char *tnmf_kernel_name(const tnmf_problem *p, int op) {
     Geo g;
     if (make_geo(p, g) || op < TNMF_OP_RECONSTRUCT || op > TNMF_OP_GRADIENT_W) return "none";
     int err;
-    const int f = choose_family(p, g, op, &err);
-    static const char *const names[3][4] = {
-        {"generic_reconstruct_kernel", "tiled::recon_kernel", "recon_tma_kernel", ""},
-        {"generic_gradient_h_kernel", "tiled::hupd_kernel", "hupd_tma_kernel", ""},
-        {"generic_gradient_w_kernel", "tiled::gradw_kernel", "gradw_tma_kernel", ""}};
-    if (f == TNMF_PATH_GENERIC) return names[op][0];
-    if (f == TNMF_PATH_TILED) return names[op][1];
-    if (f == TNMF_PATH_TMA) return names[op][2];
-    if (f != TNMF_PATH_TC) return "none";
-    if (plane_problem(g))
-        return op == TNMF_OP_RECONSTRUCT ? "recon_os3_kernel" : op == TNMF_OP_GRADIENT_H ? "hupd_ts3_kernel" : "gradw_ns3_kernel";
-    if (op == TNMF_OP_RECONSTRUCT) {
-        const int v = tc_recon_variant(p, g);
-        return v == RECON_TS ? "recon_ts_kernel" : v == RECON_OS ? "recon_os_kernel" : "recon_tc_kernel";
+    static const char *const fp32[3][3] = {   // [kernel - K_GENERIC][op]
+        {"generic_reconstruct_kernel", "generic_gradient_h_kernel", "generic_gradient_w_kernel"},
+        {"tiled::recon_kernel", "tiled::hupd_kernel", "tiled::gradw_kernel"},
+        {"recon_tma_kernel", "hupd_tma_kernel", "gradw_tma_kernel"}};
+    const int k = plan_kernel(p, g, op, &err);
+    switch (k) {
+        case K_GENERIC: case K_TILED: case K_TMA: return fp32[k - K_GENERIC][op];
+        case K_RECON_TS: return "recon_ts_kernel";
+        case K_RECON_OS: return "recon_os_kernel";
+        case K_RECON_TC: return "recon_tc_kernel";
+        case K_HUPD_TS: return "hupd_ts_kernel";
+        case K_HUPD_TC: return "hupd_tc_kernel";
+        case K_GRADW_TS: return "gradw_ts_kernel";
+        case K_GRADW_NS: return "gradw_ns_kernel";
+        case K_GRADW_TC: return "gradw_tc_kernel";
+        case K_RECON_OS3: return "recon_os3_kernel";
+        case K_HUPD_TS3: return "hupd_ts3_kernel";
+        case K_GRADW_NS3: return "gradw_ns3_kernel";
+        default: return "none";
     }
-    if (op == TNMF_OP_GRADIENT_H) return tmem_operand_hupd(g, p->dtype) ? "hupd_ts_kernel" : "hupd_tc_kernel";
-    const int v = tc_gradw_variant(p, g);
-    return v == GRADW_NS ? "gradw_ns_kernel" : v == GRADW_TS ? "gradw_ts_kernel" : "gradw_tc_kernel";
 }
 
 int tnmf_launch_count(const tnmf_problem *p, int op) {
@@ -337,13 +309,53 @@ int tnmf_launch_count(const tnmf_problem *p, int op) {
     if (make_geo(p, g)) return -1;
     if (op < TNMF_OP_RECONSTRUCT || op > TNMF_OP_GRADIENT_W) return -1;
     int err;
-    const int f = choose_family(p, g, op, &err);
-    if (f < 0) return -1;
-    if (op == TNMF_OP_GRADIENT_W)                                                            // + the finishing reduction
-        return f != TNMF_PATH_TC ? 2 : tc_gradw_variant(p, g) == GRADW_NS ? tc_gradw_ns_launches(g)
-                                     : tc_gradw_variant(p, g) == GRADW_TS ? tc_gradw_ts_launches(g) : tc_gradw_launches(g);
-    if (f == TNMF_PATH_TC) return op == TNMF_OP_RECONSTRUCT ? g.A[0] : tc_hupd_launches(g);    // (3-D: one per atom plane)
-    return f == TNMF_PATH_TMA ? 2 : 1;                                                      // + the atom pre-arrangement
+    switch (plan_kernel(p, g, op, &err)) {
+        case K_GENERIC: case K_TILED: return op == TNMF_OP_GRADIENT_W ? 2 : 1;     // + the finishing reduction
+        case K_TMA: return 2;                                   // + the atom pre-arrangement / the finishing reduction
+        case K_RECON_TS: case K_RECON_TC: return 1;
+        case K_RECON_OS: case K_RECON_OS3: return tc_recon_os_launches(g);
+        case K_HUPD_TS: case K_HUPD_TS3: return tc_hupd_ts_launches(g);
+        case K_HUPD_TC: return tc_hupd_launches(g);
+        case K_GRADW_TS: return tc_gradw_ts_launches(g);
+        case K_GRADW_NS: case K_GRADW_NS3: return tc_gradw_ns_launches(g);
+        case K_GRADW_TC: return tc_gradw_launches(g);
+        default: return -1;
+    }
+}
+
+// The reconstruction behind tnmf_reconstruct (V, partials: null) and tnmf_reconstruct_energy (the TMA kernels keep their
+// energy partials at their own place in the workspace)
+static int reconstruct_dispatch(const tnmf_problem *p, const Geo &g, int k, const void *W, const void *H, void *R,
+                                const void *V, double *&partials, int *n_partials, void *workspace,
+                                size_t workspace_bytes, cudaStream_t st) {
+    switch (k) {
+        case K_RECON_TS:
+            return tc_reconstruct_ts(g, (const float *)W, (const float *)H, (float *)R, (const float *)V, partials,
+                                     n_partials, st);
+        case K_RECON_OS3:                       // (an energy without a caller's R accumulates in workspace scratch)
+            if (!R) R = (char *)workspace + energy_partials_bytes(g);
+            [[fallthrough]];
+        case K_RECON_OS:
+            return tc_reconstruct_os(g, (const float *)W, (const float *)H, (float *)R, (const float *)V, partials,
+                                     n_partials, st);
+        case K_RECON_TC:
+            return tc_reconstruct(g, (const float *)W, (const float *)H, (float *)R, (const float *)V, partials,
+                                  n_partials, st);
+        case K_TMA:
+            if (V) partials = tma_energy_partials(g, workspace);
+            return tma_reconstruct(g, (const float *)W, (const float *)H, (float *)R, (const float *)V, partials,
+                                   n_partials, workspace, workspace_bytes, st);
+        case K_TILED:
+            return tiled_reconstruct(g, (const float *)W, (const float *)H, (float *)R, (const float *)V, partials,
+                                     n_partials, st);
+        case K_GENERIC: break;
+        default: return TNMF_EUNSUPPORTED;
+    }
+    if (p->dtype == TNMF_F32)
+        return generic_reconstruct<float>(g, (const float *)W, (const float *)H, (float *)R, (const float *)V, partials,
+                                          n_partials, st);
+    return generic_reconstruct<double>(g, (const double *)W, (const double *)H, (double *)R, (const double *)V,
+                                       partials, n_partials, st);
 }
 
 int tnmf_reconstruct(const tnmf_problem *p, const void *W, const void *H, void *R, void *workspace,
@@ -353,32 +365,11 @@ int tnmf_reconstruct(const tnmf_problem *p, const void *W, const void *H, void *
     if (s) return s;
     if (!W || !H || !R) return TNMF_EINVAL;
     if (g.N == 0) return TNMF_OK;
-    cudaStream_t st = (cudaStream_t)stream;
-    int family = choose_family(p, g, TNMF_OP_RECONSTRUCT, &s);
-    if (s) return s;
-    if (family == TNMF_PATH_TC) {
-        const int variant = tc_recon_variant(p, g);
-        if (variant == RECON_TS)
-            return tc_reconstruct_ts(g, (const float *)W, (const float *)H, (float *)R, nullptr, nullptr, nullptr, st);
-        if (variant == RECON_OS)
-            return tc_reconstruct_os(g, (const float *)W, (const float *)H, (float *)R, nullptr, nullptr, nullptr, st);
-        return tc_reconstruct(g, (const float *)W, (const float *)H, (float *)R, nullptr, nullptr, nullptr, st);
-    }
-    if (family == TNMF_PATH_TMA && (!aligned16(H) || !workspace)) {
-        if (p->path == TNMF_PATH_TMA) return workspace ? TNMF_EUNSUPPORTED : TNMF_EWORKSPACE;
-        family = tiled_supported(g, p->dtype) ? TNMF_PATH_TILED : TNMF_PATH_GENERIC;
-    }
-    if (family == TNMF_PATH_TMA)
-        return tma_reconstruct(g, (const float *)W, (const float *)H, (float *)R, nullptr, nullptr, nullptr, workspace,
-                               workspace_bytes, st);
-    const bool tiled = family == TNMF_PATH_TILED;
-    if (tiled)
-        return tiled_reconstruct(g, (const float *)W, (const float *)H, (float *)R, nullptr, nullptr, nullptr, st);
-    if (p->dtype == TNMF_F32)
-        return generic_reconstruct<float>(g, (const float *)W, (const float *)H, (float *)R, nullptr, nullptr,
-                                          nullptr, st);
-    return generic_reconstruct<double>(g, (const double *)W, (const double *)H, (double *)R, nullptr, nullptr,
-                                       nullptr, st);
+    int k = plan_kernel(p, g, TNMF_OP_RECONSTRUCT, &s);
+    if (s || (s = tma_fallback(p, g, k, aligned16(H), workspace))) return s;
+    double *partials = nullptr;
+    return reconstruct_dispatch(p, g, k, W, H, R, nullptr, partials, nullptr, workspace, workspace_bytes,
+                                (cudaStream_t)stream);
 }
 
 int tnmf_reconstruct_energy(const tnmf_problem *p, const void *V, const void *W, const void *H, void *R,
@@ -395,33 +386,9 @@ int tnmf_reconstruct_energy(const tnmf_problem *p, const void *V, const void *W,
         cudaError_t e = cudaMemsetAsync(energy, 0, sizeof(double), st);
         return status_from_cuda(e);
     }
-    int family = choose_family(p, g, TNMF_OP_RECONSTRUCT, &s);
-    if (s) return s;
-    if (family == TNMF_PATH_TMA && !aligned16(H)) {
-        if (p->path == TNMF_PATH_TMA) return TNMF_EUNSUPPORTED;
-        family = tiled_supported(g, p->dtype) ? TNMF_PATH_TILED : TNMF_PATH_GENERIC;
-    }
-    const bool tiled = family == TNMF_PATH_TILED;
-    if (family == TNMF_PATH_TC && tc_recon_variant(p, g) == RECON_TS) {
-        s = tc_reconstruct_ts(g, (const float *)W, (const float *)H, (float *)R, (const float *)V, partials, &n_partials, st);
-    } else if (family == TNMF_PATH_TC && tc_recon_variant(p, g) == RECON_OS) {
-        if (!R && plane_problem(g)) R = (char *)workspace + energy_partials_bytes(g);
-        s = tc_reconstruct_os(g, (const float *)W, (const float *)H, (float *)R, (const float *)V, partials, &n_partials, st);
-    } else if (family == TNMF_PATH_TC) {
-        s = tc_reconstruct(g, (const float *)W, (const float *)H, (float *)R, (const float *)V, partials, &n_partials, st);
-    } else if (family == TNMF_PATH_TMA) {
-        partials = tma_energy_partials(g, workspace);
-        s = tma_reconstruct(g, (const float *)W, (const float *)H, (float *)R, (const float *)V, partials, &n_partials,
-                            workspace, workspace_bytes, st);
-    } else if (tiled)
-        s = tiled_reconstruct(g, (const float *)W, (const float *)H, (float *)R, (const float *)V, partials,
-                              &n_partials, st);
-    else if (p->dtype == TNMF_F32)
-        s = generic_reconstruct<float>(g, (const float *)W, (const float *)H, (float *)R, (const float *)V, partials,
-                                       &n_partials, st);
-    else
-        s = generic_reconstruct<double>(g, (const double *)W, (const double *)H, (double *)R, (const double *)V,
-                                        partials, &n_partials, st);
+    int k = plan_kernel(p, g, TNMF_OP_RECONSTRUCT, &s);
+    if (s || (s = tma_fallback(p, g, k, aligned16(H), workspace))) return s;
+    s = reconstruct_dispatch(p, g, k, W, H, R, V, partials, &n_partials, workspace, workspace_bytes, st);
     if (s) return s;
     return finish_energy(partials, n_partials, energy, st);
 }
@@ -437,26 +404,25 @@ static int gradient_h_dispatch(const tnmf_problem *p, const void *V, const void 
     if (!V || !R || !W) return TNMF_EINVAL;
     if (g.N == 0) return TNMF_OK;
     cudaStream_t st = (cudaStream_t)stream;
-    int family = choose_family(p, g, TNMF_OP_GRADIENT_H, &s);
-    if (s) return s;
-    if (family == TNMF_PATH_TC && tmem_operand_hupd(g, p->dtype))
-        return tc_gradient_h_ts(g, (const float *)V, (const float *)R, (const float *)W, (float *)neg, (float *)pos,
-                                (float *)H, reg, (const float *)G, lambda, (const float *)Gsum, lambda_cross, st);
-    if (family == TNMF_PATH_TC)
-        return tc_gradient_h(g, (const float *)V, (const float *)R, (const float *)W, (float *)neg, (float *)pos,
-                             (float *)H, reg, (const float *)G, lambda, (const float *)Gsum, lambda_cross, st);
-    if (family == TNMF_PATH_TMA && (!aligned16(V) || !aligned16(R) || !workspace)) {
-        if (p->path == TNMF_PATH_TMA) return workspace ? TNMF_EUNSUPPORTED : TNMF_EWORKSPACE;
-        family = tiled_supported(g, p->dtype) ? TNMF_PATH_TILED : TNMF_PATH_GENERIC;
+    int k = plan_kernel(p, g, TNMF_OP_GRADIENT_H, &s);
+    if (s || (s = tma_fallback(p, g, k, aligned16(V) && aligned16(R), workspace))) return s;
+    switch (k) {
+        case K_HUPD_TS: case K_HUPD_TS3:
+            return tc_gradient_h_ts(g, (const float *)V, (const float *)R, (const float *)W, (float *)neg, (float *)pos,
+                                    (float *)H, reg, (const float *)G, lambda, (const float *)Gsum, lambda_cross, st);
+        case K_HUPD_TC:
+            return tc_gradient_h(g, (const float *)V, (const float *)R, (const float *)W, (float *)neg, (float *)pos,
+                                 (float *)H, reg, (const float *)G, lambda, (const float *)Gsum, lambda_cross, st);
+        case K_TMA:
+            return tma_gradient_h(g, (const float *)V, (const float *)R, (const float *)W, (float *)neg, (float *)pos,
+                                  (float *)H, reg, (const float *)G, lambda, (const float *)Gsum, lambda_cross,
+                                  workspace, workspace_bytes, st);
+        case K_TILED:
+            return tiled_gradient_h(g, (const float *)V, (const float *)R, (const float *)W, (float *)neg, (float *)pos,
+                                    (float *)H, reg, (const float *)G, lambda, (const float *)Gsum, lambda_cross, st);
+        case K_GENERIC: break;
+        default: return TNMF_EUNSUPPORTED;
     }
-    if (family == TNMF_PATH_TMA)
-        return tma_gradient_h(g, (const float *)V, (const float *)R, (const float *)W, (float *)neg, (float *)pos,
-                              (float *)H, reg, (const float *)G, lambda, (const float *)Gsum, lambda_cross, workspace,
-                              workspace_bytes, st);
-    const bool tiled = family == TNMF_PATH_TILED;
-    if (tiled)
-        return tiled_gradient_h(g, (const float *)V, (const float *)R, (const float *)W, (float *)neg, (float *)pos,
-                                (float *)H, reg, (const float *)G, lambda, (const float *)Gsum, lambda_cross, st);
     if (p->dtype == TNMF_F32)
         return generic_gradient_h<float>(g, (const float *)V, (const float *)R, (const float *)W, (float *)neg,
                                          (float *)pos, (float *)H, reg, (const float *)G, lambda,
@@ -499,34 +465,28 @@ int tnmf_gradient_w(const tnmf_problem *p, const void *V, const void *R, const v
         if (e == cudaSuccess) e = cudaMemsetAsync(pos, 0, count * esz, st);
         return status_from_cuda(e);
     }
-    int family = choose_family(p, g, TNMF_OP_GRADIENT_W, &s);
-    if (s) return s;
-    if (family == TNMF_PATH_TC) {
-        if (!workspace || workspace_bytes < tnmf_workspace_bytes(p)) return TNMF_EWORKSPACE;
-        const int variant = tc_gradw_variant(p, g);
-        if (variant == GRADW_NS)
+    int k = plan_kernel(p, g, TNMF_OP_GRADIENT_W, &s);
+    // every W gradient but the generic one needs the workspace, so a missing one is an error rather than a fallback
+    if (s || (s = tma_fallback(p, g, k, aligned16(V) && aligned16(R) && aligned16(H), true))) return s;
+    if (k != K_GENERIC && (!workspace || workspace_bytes < tnmf_workspace_bytes(p))) return TNMF_EWORKSPACE;
+    switch (k) {
+        case K_GRADW_NS: case K_GRADW_NS3:
             return tc_gradient_w_ns(g, (const float *)V, (const float *)R, (const float *)H, (float *)neg, (float *)pos,
                                     workspace, workspace_bytes, st);
-        if (variant == GRADW_TS)
+        case K_GRADW_TS:
             return tc_gradient_w_ts(g, (const float *)V, (const float *)R, (const float *)H, (float *)neg, (float *)pos,
                                     workspace, workspace_bytes, st);
-        return tc_gradient_w(g, (const float *)V, (const float *)R, (const float *)H, (float *)neg, (float *)pos,
-                             workspace, workspace_bytes, st);
-    }
-    if (family == TNMF_PATH_TMA && (!aligned16(V) || !aligned16(R) || !aligned16(H))) {
-        if (p->path == TNMF_PATH_TMA) return TNMF_EUNSUPPORTED;
-        family = tiled_supported(g, p->dtype) ? TNMF_PATH_TILED : TNMF_PATH_GENERIC;
-    }
-    if (family == TNMF_PATH_TMA) {
-        if (!workspace || workspace_bytes < tnmf_workspace_bytes(p)) return TNMF_EWORKSPACE;
-        return tma_gradient_w(g, (const float *)V, (const float *)R, (const float *)H, (float *)neg, (float *)pos,
-                              workspace, workspace_bytes, st);
-    }
-    const bool tiled = family == TNMF_PATH_TILED;
-    if (tiled) {
-        if (!workspace || workspace_bytes < tnmf_workspace_bytes(p)) return TNMF_EWORKSPACE;
-        return tiled_gradient_w(g, (const float *)V, (const float *)R, (const float *)H, (float *)neg, (float *)pos,
-                                workspace, workspace_bytes, st);
+        case K_GRADW_TC:
+            return tc_gradient_w(g, (const float *)V, (const float *)R, (const float *)H, (float *)neg, (float *)pos,
+                                 workspace, workspace_bytes, st);
+        case K_TMA:
+            return tma_gradient_w(g, (const float *)V, (const float *)R, (const float *)H, (float *)neg, (float *)pos,
+                                  workspace, workspace_bytes, st);
+        case K_TILED:
+            return tiled_gradient_w(g, (const float *)V, (const float *)R, (const float *)H, (float *)neg, (float *)pos,
+                                    workspace, workspace_bytes, st);
+        case K_GENERIC: break;
+        default: return TNMF_EUNSUPPORTED;
     }
     if (p->dtype == TNMF_F32)
         return generic_gradient_w<float>(g, (const float *)V, (const float *)R, (const float *)H, (float *)neg,
@@ -538,15 +498,14 @@ int tnmf_gradient_w(const tnmf_problem *p, const void *V, const void *R, const v
 // The plane-window entry points: the kernels that serve them are the plane mode of the tensor-memory kernels (3-D float32
 // 'valid') and the generic kernels; every other family has no window and the call is unsupported.  The window is on the
 // first shift axis of the problem as the caller describes it (no rows view).
-static int window_family(const tnmf_problem *p, Geo &g, int op, int t_lo, int t_hi, int *family) {
+static int window_kernel(const tnmf_problem *p, Geo &g, int op, int t_lo, int t_hi, int *k) {
     int s = make_geo(p, g, false);
     if (s) return s;
     const int wax = 3 - p->ndim;
     if (t_lo < 0 || t_hi < t_lo || t_hi > g.T[wax]) return TNMF_EINVAL;
-    *family = choose_family(p, g, op, &s);
+    *k = plan_kernel(p, g, op, &s);
     if (s) return s;
-    if (*family == TNMF_PATH_GENERIC || (*family == TNMF_PATH_TC && plane_problem(g))) return TNMF_OK;
-    return TNMF_EUNSUPPORTED;
+    return *k == K_GENERIC || *k == K_HUPD_TS3 || *k == K_GRADW_NS3 ? TNMF_OK : TNMF_EUNSUPPORTED;
 }
 
 int tnmf_update_h_planes(const tnmf_problem *p, const void *V, const void *R, const void *W, void *H, double reg,
@@ -559,12 +518,12 @@ int tnmf_update_h_planes(const tnmf_problem *p, const void *V, const void *R, co
     if (lambda == 0.0 && !Gsum) G = nullptr;
     if ((lambda != 0.0 || Gsum) && !G) return TNMF_EINVAL;
     Geo g;
-    int family;
-    int s = window_family(p, g, TNMF_OP_GRADIENT_H, t_lo, t_hi, &family);
+    int k;
+    int s = window_kernel(p, g, TNMF_OP_GRADIENT_H, t_lo, t_hi, &k);
     if (s) return s;
     if (g.N == 0 || t_lo == t_hi) return TNMF_OK;
     cudaStream_t st = (cudaStream_t)stream;
-    if (family == TNMF_PATH_TC)
+    if (k == K_HUPD_TS3)
         return tc_gradient_h_ts(g, (const float *)V, (const float *)R, (const float *)W, nullptr, nullptr, (float *)H, reg,
                                 (const float *)G, lambda, (const float *)Gsum, lambda_cross, st, t_lo, t_hi);
     if (p->dtype == TNMF_F32)
@@ -580,8 +539,8 @@ int tnmf_gradient_w_planes(const tnmf_problem *p, const void *V, const void *R, 
                            int32_t t_lo, int32_t t_hi, void *workspace, size_t workspace_bytes, void *stream) {
     if (!V || !R || !H || !neg || !pos) return TNMF_EINVAL;
     Geo g;
-    int family;
-    int s = window_family(p, g, TNMF_OP_GRADIENT_W, t_lo, t_hi, &family);
+    int k;
+    int s = window_kernel(p, g, TNMF_OP_GRADIENT_W, t_lo, t_hi, &k);
     if (s) return s;
     cudaStream_t st = (cudaStream_t)stream;
     if (g.N == 0) {
@@ -590,7 +549,7 @@ int tnmf_gradient_w_planes(const tnmf_problem *p, const void *V, const void *R, 
         if (e == cudaSuccess) e = cudaMemsetAsync(pos, 0, bytes, st);
         return status_from_cuda(e);
     }
-    if (family == TNMF_PATH_TC) {
+    if (k == K_GRADW_NS3) {
         if (!workspace || workspace_bytes < tnmf_workspace_bytes(p)) return TNMF_EWORKSPACE;
         return tc_gradient_w_ns(g, (const float *)V, (const float *)R, (const float *)H, (float *)neg, (float *)pos,
                                 workspace, workspace_bytes, st, t_lo, t_hi);

@@ -127,6 +127,7 @@ int tc_reconstruct(const Geo &g, const float *W, const float *H, float *R, const
 
 // ---- implemented in tc_hupd_ts.cu (tcgen05 3xTF32, expanded operand in tensor memory) ---------------------------
 bool tc_hupd_ts_supported(const Geo &g, int dtype);
+int tc_hupd_ts_launches(const Geo &g);
 // t_lo, t_hi: 3-D only, update the activation planes [t_lo, t_hi) only (t_hi < 0: all of them)
 int tc_gradient_h_ts(const Geo &g, const float *V, const float *R, const float *W, float *neg, float *pos, float *H,
                      double reg, const float *G, double lambda, const float *Gsum, double lambda_cross, cudaStream_t st,
@@ -141,6 +142,7 @@ int tc_reconstruct_ts(const Geo &g, const float *W, const float *H, float *R, co
 // ---- implemented in tc_recon_os.cu (tcgen05 3xTF32, narrow atoms: output-row accumulator ring in tensor memory) -------
 bool tc_recon_os_supported(const Geo &g, int dtype);
 int tc_recon_os_partials(const Geo &g);
+int tc_recon_os_launches(const Geo &g);          // one per atom plane
 int tc_reconstruct_os(const Geo &g, const float *W, const float *H, float *R, const float *V, double *energy_partials,
                       int *n_partials, cudaStream_t st);
 

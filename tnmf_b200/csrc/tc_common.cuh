@@ -51,6 +51,12 @@ struct Geo3 : tiled::Geo2 {
     long long hsz;          // element stride between activation planes (T_y * hsy)
 };
 
+// 2-D problems the tensor-core kernels serve: float32, not 'circular', rank <= 2 but not rank 1 (the FP32 kernels serve
+// that), at least one sample
+inline bool rank2_ok(const Geo &g, int dtype) {
+    if (dtype != TNMF_F32 || g.wrap || g.N < 1) return false;
+    return g.D[0] == 1 && g.A[0] == 1 && g.T[0] == 1 && !(g.D[1] == 1 && g.A[1] == 1);
+}
 // 3-D problems the plane mode serves: float32 'valid' (off = A - 1 on every axis)
 inline bool plane_mode_ok(const Geo &g, int dtype) {
     if (dtype != TNMF_F32 || g.wrap || !plane_problem(g) || g.N < 1) return false;

@@ -500,10 +500,7 @@ static bool plan_tall(const Geo2 &q, int &h, int &n) {
 }  // namespace tc
 
 bool tc_gradw_supported(const Geo &g, int dtype) {
-    if (dtype != TNMF_F32 || g.wrap) return false;
-    if (g.D[0] != 1 || g.A[0] != 1 || g.T[0] != 1) return false;      // rank <= 2
-    if (g.D[1] == 1 && g.A[1] == 1) return false;                     // rank 1: the FP32 kernels serve it
-    if (g.N < 1) return false;
+    if (!tc::rank2_ok(g, dtype)) return false;
     tc::gw::Plan p;
     const tiled::Geo2 q = tiled::make_geo2(g);
     int h, n;

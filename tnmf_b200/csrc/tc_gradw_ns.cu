@@ -491,10 +491,7 @@ __global__ void __launch_bounds__(kThreads, 1) gradw_ns3_kernel(const Geo3 g, co
 bool tc_gradw_ns_supported(const Geo &g, int dtype) {
     tc::gwn::Plan p;
     if (plane_problem(g)) return tc::plane_mode_ok(g, dtype) && tc::gwn::make_plan(tc::make_geo3(g, false), p);
-    if (dtype != TNMF_F32 || g.wrap) return false;
-    if (g.D[0] != 1 || g.A[0] != 1 || g.T[0] != 1) return false;      // rank <= 2
-    if (g.D[1] == 1 && g.A[1] == 1) return false;                     // rank 1: the FP32 kernels serve it
-    if (g.N < 1) return false;
+    if (!tc::rank2_ok(g, dtype)) return false;
     return tc::gwn::make_plan(tiled::make_geo2(g), p);
 }
 

@@ -478,10 +478,7 @@ static int launch(const Geo2 &g, const TcHupdPlan &p, const TcHupdArgs &a, cudaS
 
 // ---- dispatch ----------------------------------------------------------------------------------------------------------
 bool tc_hupd_supported(const Geo &g, int dtype) {
-    if (dtype != TNMF_F32 || g.wrap) return false;
-    if (g.D[0] != 1 || g.A[0] != 1 || g.T[0] != 1) return false;      // rank <= 2
-    if (g.D[1] == 1 && g.A[1] == 1) return false;                     // rank 1: the FP32 kernels serve it
-    if (g.N < 1) return false;
+    if (!tc::rank2_ok(g, dtype)) return false;
     tc::TcHupdPlan p;
     return tc::make_tc_hupd_plan(tiled::make_geo2(g), p);
 }

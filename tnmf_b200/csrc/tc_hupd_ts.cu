@@ -527,10 +527,7 @@ static int launch(const G &g, const Plan &p, const Args &a, cudaStream_t st) {
 bool tc_hupd_ts_supported(const Geo &g, int dtype) {
     tc::hut::Plan p;
     if (plane_problem(g)) return tc::plane_mode_ok(g, dtype) && tc::hut::make_plan(tc::make_geo3(g, true), p);
-    if (dtype != TNMF_F32 || g.wrap) return false;
-    if (g.D[0] != 1 || g.A[0] != 1 || g.T[0] != 1) return false;      // rank <= 2
-    if (g.D[1] == 1 && g.A[1] == 1) return false;                     // rank 1: the FP32 kernels serve it
-    if (g.N < 1) return false;
+    if (!tc::rank2_ok(g, dtype)) return false;
     return tc::hut::make_plan(tiled::make_geo2(g), p);
 }
 
@@ -579,5 +576,7 @@ int tc_gradient_h_ts(const Geo &g, const float *V, const float *R, const float *
     if (t_hi >= 0) return TNMF_EUNSUPPORTED;
     return gradient_h_ts(tiled::make_geo2(g), g.M, V, R, W, neg, pos, H, reg, G, lambda, Gsum, lambda_cross, st);
 }
+
+int tc_hupd_ts_launches(const Geo &g) { return tiled::ceil_div(g.M, tc::hut::kNB); }
 
 }  // namespace tnmf

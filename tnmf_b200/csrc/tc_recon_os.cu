@@ -526,10 +526,7 @@ bool tc_recon_os_supported(const Geo &g, int dtype) {
     tc::rco::Plan p;
     if (plane_problem(g))
         return g.C <= 2 && tc::plane_mode_ok(g, dtype) && tc::rco::make_plan(tc::make_geo3(g, false), p);
-    if (dtype != TNMF_F32 || g.wrap) return false;
-    if (g.D[0] != 1 || g.A[0] != 1 || g.T[0] != 1) return false;      // rank <= 2
-    if (g.D[1] == 1 && g.A[1] == 1) return false;                     // rank 1: the FP32 kernels serve it
-    if (g.N < 1 || g.C > 2) return false;
+    if (!tc::rank2_ok(g, dtype) || g.C > 2) return false;
     return tc::rco::make_plan(tiled::make_geo2(g), p);
 }
 
@@ -574,5 +571,7 @@ int tc_reconstruct_os(const Geo &g, const float *W, const float *H, float *R, co
     }
     return TNMF_OK;
 }
+
+int tc_recon_os_launches(const Geo &g) { return g.A[0]; }
 
 }  // namespace tnmf

@@ -536,10 +536,7 @@ static int launch(const Geo2 &g, const Plan &p, const Args &a, cudaStream_t st) 
 
 // ---- dispatch ----------------------------------------------------------------------------------------------------------
 bool tc_recon_ts_supported(const Geo &g, int dtype) {
-    if (dtype != TNMF_F32 || g.wrap) return false;
-    if (g.D[0] != 1 || g.A[0] != 1 || g.T[0] != 1) return false;      // rank <= 2
-    if (g.D[1] == 1 && g.A[1] == 1) return false;                     // rank 1: the FP32 kernels serve it
-    if (g.N < 1 || g.C > 4) return false;
+    if (!tc::rank2_ok(g, dtype) || g.C > 4) return false;
     tc::rct::Plan p;
     return tc::rct::make_plan(tiled::make_geo2(g), p);
 }
