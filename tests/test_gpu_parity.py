@@ -612,6 +612,8 @@ OS_CASES = [
     (40, 1, 17, (20, 130), (15, 3)),    # more work units than SMs; 17 atoms padded to 24
     (2, 2, 30, (64, 40), (7, 12)),      # 32-column slots: ring of 10, three stages
     (1, 1, 32, (15, 15), (15, 15)),     # atom as large as the sample ('full': one activation feeds every output row)
+    (160, 1, 32, (16, 128), (15, 15)),  # 200 tiles, 22 rows per CTA: a CTA's range spans whole tiles (up to 3 segments);
+                                        # 'full': a segment's last source row completes 10 rows, the next opens 15
 ]
 
 

@@ -372,23 +372,34 @@ __device__ __forceinline__ void recon_os_body(const G &g, const Plan &p, const A
         // the kernel).  The loop is therefore SOFTWARE-PIPELINED: the books and the waits of source row i + 1 are done
         // after all but the last K step of row i have been issued - under MMAs that are executing or queued - and only
         // then follow the last K step of row i and its commits.
+        // A slot is waited for (d_free) in `prep` only when the row it held was committed before: prep of source row i + 1
+        // runs before the commits of row i, and where row i completes many output rows at once (the bottom of a 'full'
+        // problem) while row i + 1 opens the next segment with up to A_y rows, the slot can hold a row that row i
+        // completes - waiting for it there would never return.  Such waits follow the commits of row i (`wait_late`).
         struct Row {
             bool valid;
             int st, second, done;                               // operand stage, rows past the ring's wrap, rows this row completes
+            int n_late, late_slot;                              // entering rows whose slots are waited for after the commits
+            unsigned late_wraps;
             unsigned d0, bo, bo1, idesc0, idesc1, ta_hi, ta_lo;
         };
         long long u = blockIdx.x;
         Unit w = make_unit(u, g, p);
         bool in_unit = u < p.units && w.y0 < w.y1;
         int ty = w.ta, next_in = w.y0, win_lo = w.y0, next_out = w.y0;
+        long long rows_in = 0, rows_out = 0;                    // output rows of this CTA entered / committed so far
         auto prep = [&]() {
             Row r;
             r.valid = in_unit;
+            r.n_late = 0;
             if (!in_unit) return r;
             const int yhi = min(w.y1 - 1, ty - g.offy + AY - 1), ylo = max(w.y0, ty - g.offy);
             // output rows that enter the window with this source row: their slots must have been drained
-            for (; next_in <= yhi; ++next_in) {
-                if (wraps_in) TC_PROF_WAIT(dfree, mbar_wait(&d_free[slot_in], (wraps_in - 1u) & 1u));
+            for (; next_in <= yhi; ++next_in, ++rows_in) {
+                if (wraps_in) {
+                    if (rows_in - RSD < rows_out) TC_PROF_WAIT(dfree, mbar_wait(&d_free[slot_in], (wraps_in - 1u) & 1u));
+                    else if (r.n_late++ == 0) { r.late_slot = slot_in; r.late_wraps = wraps_in; }
+                }
                 if (++slot_in == RSD) { slot_in = 0; ++wraps_in; }
             }
             for (; win_lo < ylo; ++win_lo)
@@ -448,7 +459,18 @@ __device__ __forceinline__ void recon_os_body(const G &g, const Plan &p, const A
                     }
             }
         };
+        auto wait_late = [&](const Row &r) {
+            if (!r.n_late) return;
+            int s = r.late_slot;
+            unsigned wr = r.late_wraps;
+            for (int i = 0; i < r.n_late; ++i) {
+                TC_PROF_WAIT(dfree, mbar_wait(&d_free[s], (wr - 1u) & 1u));
+                if (++s == RSD) { s = 0; ++wr; }
+            }
+            tc_fence_after();
+        };
         Row cur = prep();
+        wait_late(cur);
         while (cur.valid) {
 #ifdef TNMF_TC_PROFILE
             const long long t_i = clock64();
@@ -472,6 +494,8 @@ __device__ __forceinline__ void recon_os_body(const G &g, const Plan &p, const A
                 mma_commit_elect(&d_full[slot_out]);
                 if (++slot_out == RSD) slot_out = 0;
             }
+            rows_out += cur.done;
+            wait_late(nxt);
             cur = nxt;
         }
 #ifdef TNMF_TC_PROFILE
