@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define TNMF_ABI_VERSION 6
+#define TNMF_ABI_VERSION 7
 #define TNMF_MAX_SHIFT_DIMS 3
 
 /* element types */
@@ -181,6 +181,21 @@ int tnmf_update_h_planes(const tnmf_problem *p, const void *V, const void *R, co
 int tnmf_gradient_w_planes(const tnmf_problem *p, const void *V, const void *R, const void *H,
                            void *neg, void *pos, int32_t t_lo, int32_t t_hi,
                            void *workspace, size_t workspace_bytes, void *stream);
+
+/* Kullback-Leibler divergence (DESIGN.md §3.11).  For the n_samples * C * prod(D) elements of V and R (contiguous, the
+ * layout of the reconstruction):  R <- Q = V / max(R, tau), and Q = 0 where V = 0, with tau the smallest normal number
+ * of the dtype and IEEE division.  If `divergence` (a double in device memory) is non-null it receives
+ *     D(V||R) = sum [ V log(V / max(R, tau)) - V + R ]      (0 log 0 = 0)
+ * of the R passed in, each term computed in double and summed in a fixed order (per-block partials in `workspace`,
+ * tnmf_kl_workspace_bytes bytes, then one finishing kernel): bitwise reproducible.  Without `divergence` the workspace is
+ * not used.  One kernel launch, two with `divergence`.
+ * The KL multiplicative updates are the fused Frobenius calls with other inputs: tnmf_update_h(Q, ones, W, H, ...) and
+ * tnmf_gradient_w(Q, ones, H, ...), where ones is a V-shaped tensor of ones, give neg = corr(Q) and pos = corr(ones),
+ * whose difference pos - neg is the gradient of D.
+ * TNMF_EINVAL for null V / R or a malformed problem, TNMF_EWORKSPACE for a missing or short workspace with `divergence`. */
+size_t tnmf_kl_workspace_bytes(const tnmf_problem *p);
+int tnmf_kl_quotient(const tnmf_problem *p, const void *V, void *R, double *divergence, void *workspace,
+                     size_t workspace_bytes, void *stream);
 
 /* W = (W * neg) / (pos + eps);  W[m,c,:] /= sum_a W[m,c,a].  In place; neg/pos are left untouched.
  * Replaces TransformInvariantNMF._update_W's arithmetic, tnmf/TransformInvariantNMF.py:217-244, and

@@ -15,11 +15,11 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 LIB_PATH = os.environ.get('TNMF_LIB_PATH') or os.path.join(HERE, 'libtnmf_b200.so')      # override: experiments only
 SOURCES = ('capi.cu', 'generic_kernels.cu', 'elementwise.cu', 'tiled_kernels.cu', 'tma_kernels.cu', 'tc_hupd.cu', 'tc_gradw.cu', 'tc_recon.cu',
-           'tc_gradw_ts.cu', 'tc_recon_ts.cu', 'tc_hupd_ts.cu', 'tc_recon_os.cu', 'tc_gradw_ns.cu', 'peer_update_w.cu')
+           'tc_gradw_ts.cu', 'tc_recon_ts.cu', 'tc_hupd_ts.cu', 'tc_recon_os.cu', 'tc_gradw_ns.cu', 'peer_update_w.cu', 'kl.cu')
 # compiled once per atom-width chunk (-DTNMF_AXC=...): the register-tiled kernels
 CHUNKED_SOURCES = ('tiled_recon.cu', 'tiled_hupd.cu', 'tiled_gradw.cu', 'tma_recon.cu', 'tma_hupd.cu', 'tma_gradw.cu')
 CHUNKS = (4, 8, 12, 16)
-HEADERS = ('common.cuh', 'tiled_common.cuh', 'tma_common.cuh', 'tc_common.cuh', os.path.join('..', '..', 'include', 'tnmf_b200.h'))
+HEADERS = ('common.cuh', 'tiled_common.cuh', 'tma_common.cuh', 'tc_common.cuh', 'kl.cuh', os.path.join('..', '..', 'include', 'tnmf_b200.h'))
 
 # NB: no --use_fast_math: divisions must round like the reference's IEEE arithmetic.
 NVCC_FLAGS = ('-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
@@ -30,7 +30,7 @@ MODES = {'valid': 0, 'full': 1, 'circular': 2}
 PATHS = {'auto': 0, 'generic': 1, 'tiled': 2, 'tma': 3, 'tc': 4}
 OP_RECONSTRUCT, OP_GRADIENT_H, OP_GRADIENT_W = 0, 1, 2
 TNMF_OK, TNMF_EINVAL, TNMF_EUNSUPPORTED, TNMF_EWORKSPACE, TNMF_ECUDA = 0, 1, 2, 3, 1000
-ABI_VERSION = 6
+ABI_VERSION = 7
 # tnmf_problem.flags (include/tnmf_b200.h)
 FLAG_NO_ROWS_VIEW, FLAG_ROWS_VIEW_ALWAYS = 1, 2
 FLAG_NO_TC_HUPD, FLAG_NO_TC_RECON, FLAG_NO_TC_GRADW, FLAG_NO_TC, FLAG_NO_TMA, FLAG_NO_TMEM_OPERAND = 4, 8, 16, 28, 32, 64
@@ -76,6 +76,8 @@ SIGNATURES = {
     'tnmf_gradient_w': (ctypes.c_int, [_P, _vp, _vp, _vp, _vp, _vp, _vp, _sz, _vp]),
     'tnmf_update_h_planes': (ctypes.c_int, [_P, _vp, _vp, _vp, _vp, _dbl, _vp, _dbl, _vp, _dbl, _i32, _i32, _vp, _sz, _vp]),
     'tnmf_gradient_w_planes': (ctypes.c_int, [_P, _vp, _vp, _vp, _vp, _vp, _i32, _i32, _vp, _sz, _vp]),
+    'tnmf_kl_workspace_bytes': (_sz, [_P]),
+    'tnmf_kl_quotient': (ctypes.c_int, [_P, _vp, _vp, _vp, _vp, _sz, _vp]),
     'tnmf_update_w': (ctypes.c_int, [_P, _vp, _vp, _vp, _dbl, _vp]),
     'tnmf_peer_buffer_bytes': (_sz, [_P, _i32]),
     'tnmf_allreduce_update_w': (ctypes.c_int, [_P, _vp, _vp, ctypes.POINTER(PeerWorld), _vp, _dbl, _vp]),

@@ -134,7 +134,9 @@ class B200_Backend(Backend):  # pylint: disable=invalid-name
         self._ws = None
         self.buffers_epoch = 0  # bumped whenever one of the buffers above is replaced (captured CUDA graphs watch it)
         self._energy_buf = None
-        self._R_token = None    # (W pointer, H pointer, samples) whose reconstruction `energy(keep_R=True)` left in _R_buf
+        self._R_token = None    # (W pointer, H pointer, samples, divergence) whose reconstruction `energy(keep_R=True)` left
+                                # in _R_buf ('kl': the quotient V / R in its place)
+        self._ones = None       # V-shaped tensor of ones: the second operand of the KL correlations (`divergence='kl'`)
         self._problems = {}
         self._taps = {}
         self._last_h_problem = None
@@ -260,8 +262,9 @@ class B200_Backend(Backend):  # pylint: disable=invalid-name
             buf.uniform_().neg_().add_(1)       # 1 - U[0, 1), like tnmf/backends/_Backend.py:92
         return buf[..., :shape[-1]] if pad else buf
 
-    def _workspace(self, p: _lib.Problem) -> Tuple[torch.Tensor, int]:
-        need = getattr(p, 'ws_need', None)
+    def _workspace(self, p: _lib.Problem, need: Optional[int] = None) -> Tuple[torch.Tensor, int]:
+        if need is None:
+            need = getattr(p, 'ws_need', None)
         if need is None:
             need = p.ws_need = int(self._lib.tnmf_workspace_bytes(ctypes.byref(p)))
         if self._ws is None or self._ws.numel() < need:
@@ -278,10 +281,11 @@ class B200_Backend(Backend):  # pylint: disable=invalid-name
         self._R_token = None            # whoever asks for the buffer is about to write it
         return self._R_buf[:numel].view(shape)
 
-    def holds_R_of(self, W: torch.Tensor, H: torch.Tensor) -> bool:
-        """True while the R buffer holds the reconstruction an `energy(..., keep_R=True)` call computed from exactly these
-        tensors and no other operation has written the buffer since (the caller vouches that W and H did not change)."""
-        return self._R_token is not None and self._R_token == (W.data_ptr(), H.data_ptr(), int(H.shape[0]))
+    def holds_R_of(self, W: torch.Tensor, H: torch.Tensor, divergence: str = 'frobenius') -> bool:
+        """True while the R buffer holds the reconstruction (under 'kl': the quotient V / R) an `energy(..., keep_R=True)`
+        call of this divergence computed from exactly these tensors and no other operation has written the buffer since
+        (the caller vouches that W and H did not change)."""
+        return self._R_token is not None and self._R_token == (W.data_ptr(), H.data_ptr(), int(H.shape[0]), divergence)
 
     def min_of_V(self) -> torch.Tensor:
         """Smallest element of the device copy of the samples (a device scalar; the facade's non-negativity assert)."""
@@ -289,7 +293,7 @@ class B200_Backend(Backend):  # pylint: disable=invalid-name
 
     def buffer_tensors(self) -> tuple:
         """The scratch buffers kernels of this backend write to (kept alive by whoever captured their addresses)."""
-        return tuple(t for t in (self._ws, self._R_buf, self._H_store) if t is not None)
+        return tuple(t for t in (self._ws, self._R_buf, self._H_store, self._ones) if t is not None)
 
     def buffer_pointers(self) -> tuple:
         return tuple(t.data_ptr() for t in self.buffer_tensors())
@@ -494,13 +498,52 @@ class B200_Backend(Backend):  # pylint: disable=invalid-name
 
     # -----------------------------------------------------------------------------------------------
     # fused entry points used by tnmf_b200.TransformInvariantNMF
+    #
+    # `divergence='kl'` (DESIGN.md §3.11): the generalised Kullback-Leibler divergence D(V||R) instead of 0.5*||V - R||^2.
+    # Its gradients are the Frobenius ones with (Q, ones) in place of (V, R), Q = V / R: so the same fused kernels run,
+    # after one elementwise pass (tnmf_kl_quotient) turns the reconstruction in the R buffer into Q.
     # -----------------------------------------------------------------------------------------------
-    def energy(self, V, W, H, s: slice = sliceNone, keep_R: bool = False) -> torch.Tensor:
+    @staticmethod
+    def _is_kl(divergence: str) -> bool:
+        if divergence not in ('frobenius', 'kl'):
+            raise ValueError(f'divergence must be "frobenius" or "kl" (got {divergence!r})')
+        return divergence == 'kl'
+
+    def _ones_for(self, V_full: torch.Tensor) -> torch.Tensor:
+        """Ones shaped like the device copy of the samples; minibatches slice it like V."""
+        if self._ones is None or self._ones.shape != V_full.shape or self._ones.dtype != self._dtype:
+            self._ones = None
+            self._ones = torch.ones(V_full.shape, dtype=self._dtype, device=self.device)
+            self.buffers_epoch += 1
+        return self._ones
+
+    def _kl_quotient(self, Vs: torch.Tensor, R: torch.Tensor, divergence: Optional[torch.Tensor] = None) -> None:
+        """R <- V / max(R, tau) in place (0 where V == 0); the divergence of the R passed in goes to `divergence`."""
+        p = self._problem(int(R.shape[0]), self.n_atoms)
+        need = getattr(p, 'kl_ws_need', None)
+        if need is None:
+            need = p.kl_ws_need = int(self._lib.tnmf_kl_workspace_bytes(ctypes.byref(p)))
+        ws, ws_bytes = self._workspace(p, need)
+        with self._timed('kl_quotient'):
+            _lib.check(self._lib.tnmf_kl_quotient(ctypes.byref(p), Vs.data_ptr(), R.data_ptr(),
+                                                  None if divergence is None else divergence.data_ptr(), ws.data_ptr(),
+                                                  ws_bytes, _stream_ptr(self.device)), 'kl_quotient')
+        self.launches += 1 if divergence is None else 2
+
+    def energy(self, V, W, H, s: slice = sliceNone, keep_R: bool = False, divergence: str = 'frobenius') -> torch.Tensor:
         """Device-resident double scalar 0.5*||V[s] - reconstruct(W, H[s])||^2 (no host synchronisation).  With `keep_R`
-        the reconstruction is also written to the R buffer, where `update_H(..., reuse_R=True)` picks it up."""
+        the reconstruction is also written to the R buffer, where `update_H(..., reuse_R=True)` picks it up.
+        `divergence='kl'`: D(V[s] || reconstruct(W, H[s])); the R buffer then holds the quotient V / R."""
         Hs = H[s]
         Vs = self._device_V(V)[s]
         keep_R = keep_R and Hs.shape[0] > 0 and Hs.data_ptr() == H.data_ptr() and Hs.shape[0] == H.shape[0]
+        if self._is_kl(divergence):
+            e = torch.empty((), dtype=torch.float64, device=self.device)
+            R = self.reconstruct(W, Hs, out=self._R_for(Hs.shape[0]))
+            self._kl_quotient(Vs, R, e)
+            if keep_R:
+                self._R_token = (W.data_ptr(), Hs.data_ptr(), int(Hs.shape[0]), divergence)
+            return e
         R = self._R_for(Hs.shape[0]) if keep_R else None
         p, Hs = self._h_problem(Hs)
         ws, ws_bytes = self._workspace(p)
@@ -510,7 +553,7 @@ class B200_Backend(Backend):  # pylint: disable=invalid-name
                                                      ws_bytes, _stream_ptr(self.device)), 'reconstruct_energy')
         self.launches += 1 + self._n_launches(p, _lib.OP_RECONSTRUCT)
         if keep_R:
-            self._R_token = (W.data_ptr(), Hs.data_ptr(), int(Hs.shape[0]))
+            self._R_token = (W.data_ptr(), Hs.data_ptr(), int(Hs.shape[0]), divergence)
         return e
 
     def _inhibition_taps(self, kernels: Sequence[np.ndarray]):
@@ -523,21 +566,28 @@ class B200_Backend(Backend):  # pylint: disable=invalid-name
 
     def update_H(self, V, W, H, s: slice = sliceNone, sparsity: float = 0., inhibition: float = 0.,
                  cross_inhibition: float = 0., inhibition_kernels: Optional[Sequence[np.ndarray]] = None,
-                 eps: float = 1.e-9, reuse_R: bool = False, planes: Optional[Tuple[int, int]] = None) -> None:
+                 eps: float = 1.e-9, reuse_R: bool = False, planes: Optional[Tuple[int, int]] = None,
+                 divergence: str = 'frobenius') -> None:
         """One in-place multiplicative update of H[s]: reconstruct, both correlations, sparsity / inhibition terms and
         H <- (H*neg)/pos in one fused kernel   (tnmf/TransformInvariantNMF.py:246-271 + :217-235).
         `planes=(t_lo, t_hi)` updates only those activation indices along the first shift axis (tnmf_update_h_planes:
         three shift axes, or any problem on the generic kernels); the reconstruction and the inhibition terms still see
-        all of H."""
+        all of H.  `divergence='kl'`: the KL update, the same kernel on (V / R, ones) instead of (V, R)."""
+        kl = self._is_kl(divergence)
         Hs = H[s]
         if Hs.shape[0] == 0:
             return
-        Vs = self._device_V(V)[s]
+        V_full = self._device_V(V)
+        Vs = V_full[s]
         n = Hs.shape[0]
-        have_R = reuse_R and self.holds_R_of(W, Hs)     # left in the buffer by `energy(keep_R=True)` for these very W, H
+        have_R = reuse_R and self.holds_R_of(W, Hs, divergence)    # left by `energy(keep_R=True)` for these very W, H
         R = self._R_for(n)                              # (clears the token: H changes below)
         if not have_R:
             R = self.reconstruct(W, Hs, out=R)
+            if kl:
+                self._kl_quotient(Vs, R)
+        if kl:
+            Vs, R = R, self._ones_for(V_full)[s]
         p, Hs = self._h_problem(Hs)
         G_ptr, Gsum_ptr = None, None
         lam, lam_cross = 0.0, 0.0
@@ -581,20 +631,26 @@ class B200_Backend(Backend):  # pylint: disable=invalid-name
         self.launches += self._n_launches(p, _lib.OP_GRADIENT_H)
 
     def gradient_W(self, V, W, H, s: slice, out: torch.Tensor, H_for_R: Optional[torch.Tensor] = None,
-                   planes: Optional[Tuple[int, int]] = None) -> torch.Tensor:
+                   planes: Optional[Tuple[int, int]] = None, divergence: str = 'frobenius') -> torch.Tensor:
         """out[0] = neg, out[1] = pos of the W gradient on samples s (split-K + deterministic final reduction).
         `H_for_R`: reconstruct from these activations instead of H (halo sharding correlates with a band of H - the other
         rows zeroed - against the reconstruction of all of it; tnmf_b200/halo.py).
         `planes=(t_lo, t_hi)`: correlate with those activation indices along the first shift axis only, as if H were zero
-        elsewhere, against the reconstruction of all of H (tnmf_gradient_w_planes; the same kernels as `update_H`'s)."""
+        elsewhere, against the reconstruction of all of H (tnmf_gradient_w_planes; the same kernels as `update_H`'s).
+        `divergence='kl'`: the KL gradient, the same kernel on (V / R, ones) instead of (V, R)."""
+        kl = self._is_kl(divergence)
         Hs = H[s]
-        Vs = self._device_V(V)[s]
+        V_full = self._device_V(V)
+        Vs = V_full[s]
         n = Hs.shape[0]
         p, Hs = self._h_problem(Hs)
         if n == 0:
             out.zero_()
             return out
         R = self.reconstruct(W, Hs if H_for_R is None else H_for_R[s], out=self._R_for(n))
+        if kl:
+            self._kl_quotient(Vs, R)
+            Vs, R = R, self._ones_for(V_full)[s]
         if H_for_R is not None:
             p, Hs = self._h_problem(Hs)         # (reconstruct recorded the other tensor's problem)
         ws, ws_bytes = self._workspace(p)

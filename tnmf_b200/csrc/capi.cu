@@ -4,6 +4,7 @@
 #include <cstdlib>
 #include <cstring>
 #include "common.cuh"
+#include "kl.cuh"
 
 using namespace tnmf;
 
@@ -559,6 +560,26 @@ int tnmf_gradient_w_planes(const tnmf_problem *p, const void *V, const void *R, 
                                          (float *)pos, st, t_lo, t_hi);
     return generic_gradient_w<double>(g, (const double *)V, (const double *)R, (const double *)H, (double *)neg,
                                       (double *)pos, st, t_lo, t_hi);
+}
+
+size_t tnmf_kl_workspace_bytes(const tnmf_problem *p) {
+    Geo g;
+    if (make_geo(p, g, false)) return 0;
+    return kl_workspace_bytes((long long)g.N * g.C * vol3(g.D));
+}
+
+int tnmf_kl_quotient(const tnmf_problem *p, const void *V, void *R, double *divergence, void *workspace,
+                     size_t workspace_bytes, void *stream) {
+    Geo g;
+    int s = make_geo(p, g, false);
+    if (s) return s;
+    if (!V || !R) return TNMF_EINVAL;
+    const long long n = (long long)g.N * g.C * vol3(g.D);
+    if (divergence && (!workspace || workspace_bytes < kl_workspace_bytes(n))) return TNMF_EWORKSPACE;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (n == 0) return divergence ? status_from_cuda(cudaMemsetAsync(divergence, 0, sizeof(double), st)) : TNMF_OK;
+    if (p->dtype == TNMF_F32) return kl_quotient<float>((const float *)V, (float *)R, n, divergence, workspace, st);
+    return kl_quotient<double>((const double *)V, (double *)R, n, divergence, workspace, st);
 }
 
 int tnmf_update_w(const tnmf_problem *p, void *W, const void *neg, const void *pos, double eps, void *stream) {

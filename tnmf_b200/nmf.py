@@ -36,7 +36,7 @@ class MiniBatchAlgorithm(Enum):
 class TransformInvariantNMF:
     r"""
     Shift-invariant non-negative matrix factorisation  V[n,c,:] ~ sum_m W[m,c,:] * H[n,m,:]  by multiplicative
-    updates on the Frobenius energy, on one or several B200 GPUs.
+    updates on the Frobenius energy or the Kullback-Leibler divergence, on one or several B200 GPUs.
 
     Parameters (first six as in tnmf/TransformInvariantNMF.py:142-151)
     ----------
@@ -61,6 +61,11 @@ class TransformInvariantNMF:
         Batch algorithm only: after one eager iteration the kernel launches of an iteration are captured into CUDA
         graphs (everything up to the all-reduce of the W gradient, and the W update after it) and replayed, which
         removes the host-side launch cost (about 1 ms of a 4.6 ms iteration on cfg2).  Results are bit-identical.
+    divergence : 'frobenius' (default) | 'kl'
+        The loss the updates minimise: 0.5*||V - R||^2, or the generalised Kullback-Leibler divergence
+        D(V||R) = sum V log(V/R) - V + R (Lee & Seung's KL updates; DESIGN.md §3.11), the usual loss for counts and
+        magnitudes.  `energy_device()` and the energy of the progress log report the chosen loss.  'kl' needs
+        `fused=True`.
     **kwargs : forwarded to `B200_Backend` (reconstruction_mode, device, init, kernel_path)
     """
 
@@ -68,7 +73,15 @@ class TransformInvariantNMF:
                  backend: str = 'b200', logger: logging.Logger = None, verbose: int = 0,
                  distributed: Optional[bool] = None, process_group=None, input_is_local_shard: bool = False,
                  fused: bool = True, cuda_graph: bool = True, equal_shards: bool = False, peer_exchange: bool = True,
-                 **kwargs):
+                 divergence: str = 'frobenius', **kwargs):
+        if divergence not in ('frobenius', 'kl'):
+            raise ValueError(f'divergence must be "frobenius" or "kl" (got {divergence!r})')
+        if divergence == 'kl' and not fused:
+            raise ValueError('divergence="kl" needs fused=True (the unfused mode is the Frobenius call sequence of the '
+                             'reference facade)')
+        self._divergence = divergence
+        # the backend hears of the divergence only when it is not the default
+        self._div_kw = {} if divergence == 'frobenius' else {'divergence': divergence}
         self.atom_shape = tuple(atom_shape)
         if inhibition_range is None:
             self._inhibition_range = tuple(a - 1 for a in self.atom_shape)   # just covers the atom
@@ -150,11 +163,12 @@ class TransformInvariantNMF:
         return self._backend.reconstruct(self._W, self._H)
 
     def energy_device(self) -> torch.Tensor:
-        """0.5*||V-R||^2 over all samples of all ranks as a device-resident double (no host sync).  The reconstruction it
+        """0.5*||V-R||^2 (with divergence='kl': D(V||R)) over all samples of all ranks as a device-resident double (no host
+        sync).  The reconstruction it
         is computed from stays in the backend's R buffer: it is the one the next H update opens with, so an energy read
         in every iteration (a progress callback, the INFO log line of tnmf/TransformInvariantNMF.py:346) costs no third
         reconstruction per iteration."""
-        e = self._backend.energy(self._V, self._W, self._H, keep_R=self._fused)
+        e = self._backend.energy(self._V, self._W, self._H, keep_R=self._fused, **self._div_kw)
         self._R_current = self._fused
         return self._sharding.sum_scalar(e)
 
@@ -181,7 +195,8 @@ class TransformInvariantNMF:
         self._R_current = False
         if self._fused:
             self._backend.update_H(self._V, self._W, self._H, s, sparsity, inhibition, cross_inhibition,
-                                   self._inhibition_kernels_1D, self.eps, reuse_R=reuse_R and s is sliceNone)
+                                   self._inhibition_kernels_1D, self.eps, reuse_R=reuse_R and s is sliceNone,
+                                   **self._div_kw)
             return
         # reference call sequence, tnmf/TransformInvariantNMF.py:246-271
         neg, pos = self._backend.reconstruction_gradient_H(self._V, self._W, self._H, s)
@@ -203,7 +218,7 @@ class TransformInvariantNMF:
     def _gradient_W(self, s: slice = sliceNone, reduce: bool = True) -> torch.Tensor:
         """Stacked (neg, pos) of the W gradient on local samples s, summed over ranks when `reduce`."""
         if self._fused:
-            grad = self._backend.gradient_W(self._V, self._W, self._H, s, self._grad)
+            grad = self._backend.gradient_W(self._V, self._W, self._H, s, self._grad, **self._div_kw)
         else:
             neg, pos = self._backend.reconstruction_gradient_W(self._V, self._W, self._H, s)
             assert neg.shape == self._W.shape and pos.shape == self._W.shape
@@ -319,7 +334,7 @@ class TransformInvariantNMF:
 
         def take_R():           # True once after an energy evaluation left the current reconstruction behind
             have, self._R_current = self._R_current and update_H, False
-            return have and self._backend.holds_R_of(self._W, self._H)
+            return have and self._backend.holds_R_of(self._W, self._H, **self._div_kw)
 
         def back():             # the W update proper (with the sum over ranks inside when the peers are mapped)
             if update_W and self._peer is not None:
@@ -340,7 +355,7 @@ class TransformInvariantNMF:
         if self._step_cache is None:
             self._step_cache = {}
         key = (bool(update_H), bool(update_W), float(sparsity), float(inhibition), float(cross_inhibition),
-               tuple(self._H.shape), tuple(self._H.stride()))
+               tuple(self._H.shape), tuple(self._H.stride()), self._divergence)
         return _GraphedStep(self._backend, front, reduce, back, self._sharding, self._step_cache, key,
                             (self._H, self._backend._device_V(self._V), self._W, self._grad), take_R)   # pylint: disable=protected-access
 
